@@ -397,10 +397,37 @@ def run_ours(args):
                                 "sample": f"{n_inst} C2 instances (seeds 0..{n_inst - 1}), oracle model + HiGHS capped at 15 s each, "
                                           f"{sum(r['optimal'] for r in recs)}/{n_inst} proven optimal inside the cap",
                                 "quality_at_cap": cpu_quality(recs)}
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(last, args.dump_outputs)
     if rank == 0:
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(res, out_dir):
+    """What the last timed step returned to its caller, one float64 `<name>.npy` per array: placement `c`, routing `x`,
+    node counts `n`, check `flags`, `scores`, the PDHG records as `lp_<field>` and the search round `lns_round`.  Every
+    array has the instance as its first axis; when they would exceed DUMP_BYTES together, a seeded sample of instances is
+    kept, and `instances.npy` always lists the instances written."""
+    arrays = {"c": res.c, "x": res.x, "n": res.n, "flags": res.flags, "scores": res.scores}
+    if res.lp is not None:
+        arrays.update({f"lp_{k}": res.lp[k] for k in res.lp.dtype.names if k != "pad"})
+    if res.lns_round is not None:
+        arrays["lns_round"] = res.lns_round
+    arrays = {k: (v.cpu().numpy() if hasattr(v, "cpu") else np.asarray(v)).astype(np.float64) for k, v in arrays.items()}
+    B = len(arrays["c"])
+    per_instance = sum(v.nbytes for v in arrays.values()) // B
+    keep = np.arange(B)
+    if per_instance * B > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(B, DUMP_BYTES // per_instance, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "instances.npy"), keep.astype(np.float64))
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v[keep])
 
 
 def c5_sweep(args, rank, world, barrier):
@@ -503,7 +530,13 @@ def main():
     ap.add_argument("--c4-iters", type=int, default=64)
     ap.add_argument("--ref-limit", type=float, default=20.0, help="--impl reference: HiGHS cap per instance (s)")
     ap.add_argument("--ref-instances", type=int, default=0, help="--impl reference: instances per step (0 = one per worker)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0's instances) as DIR/<name>.npy, at most 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,5 +1,5 @@
-"""TEST INFRASTRUCTURE ONLY -- regenerate tests/golden/*.json.  Run in the build container only
-(/root/reference must exist):   python -m oracle.make_golden [--only NAME] [--jobs J]
+"""TEST INFRASTRUCTURE ONLY -- regenerate tests/golden/*.json:   python -m oracle.make_golden [--only NAME] [--jobs J]
+The steps that run the unmodified reference need its tree (oracle/refshim, NEPTUNE_REFERENCE_ROOT).
 
 Sources of truth written into the fixtures
   alibaba_case0.json   the reference's own shipped outputs testing/alibaba/alibaba_test/output_*_case0.json
@@ -15,6 +15,8 @@ Sources of truth written into the fixtures
   payload_json.json    the reference's payload.json sample (no matrices: every default) through six solvers
   mip_optima.json      step-1 optima by HiGHS on the oracle model (C2 seeds, C5 subsample), with the placements
   lp_cut.json          HiGHS optima of the slot-cut LP relaxation (oracle.relax) the matrix-free PDHG solves
+  reference_vectors.json  input-adapter arrays, response shaping, step-1 matrix digests and EFTTC results on the small
+                       payloads of tests/helpers.py (see make_reference_vectors)
 """
 from __future__ import annotations
 
@@ -37,10 +39,10 @@ GOLD = os.path.join(ROOT, "tests", "golden")
 REF = "/root/reference"
 
 
-def _dump(name, obj):
+def _dump(name, obj, indent=1):
     os.makedirs(GOLD, exist_ok=True)
     with open(os.path.join(GOLD, name), "w") as fh:
-        json.dump(obj, fh, indent=1, sort_keys=True)
+        json.dump(obj, fh, indent=indent, sort_keys=True)
     print("wrote", name)
 
 
@@ -272,6 +274,45 @@ def make_mip_optima(jobs, c2_seeds=16, c5_seeds=64):
             _dump("mip_optima.json", sorted(have.values(), key=lambda r: (r["config"], r["kind"], r["seed"])))
 
 
+def make_reference_vectors():
+    """What tests/test_oracle_vs_reference.py and the edge-case test of tests/test_host_logic.py hold the project to, on
+    the payloads of tests/helpers.py: the input adapter's arrays, the response shaping of a seeded random solution,
+    digests of the step-1 matrices and the EFTTC results (strict, and with the `discard` fallback).  Those tests used to
+    import the unmodified reference and require equality with it; these values are computed by the project's
+    restatements (core.utils adapter, core.solvers.output, oracle.model, oracle.efttc) as they stood when those tests
+    held them equal to the reference, so that the comparison no longer needs the reference tree."""
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from helpers import DATA_FIELDS, arrays_of, data_of, edge_payloads, shaping_solution, small_payloads
+    from neptune_mip_b200.core.solvers.output import convert_c_matrix, convert_x_matrix
+    from oracle import efttc, model
+    out = {"data": {}, "shaping": {}, "model": {}, "efttc": {}}
+    edges = edge_payloads()
+    for name, p in [(n, p) for n, p, _ in small_payloads()] + list(edges.items()):
+        d = data_of(p)
+        out["data"][name] = dict({k: np.asarray(getattr(d, k)).tolist() for k in DATA_FIELDS},
+                                 nodes=d.nodes, functions=d.functions, node_budget=_np_to_py(d.node_budget))
+        if name in edges:
+            x, c = shaping_solution(len(d.nodes), len(d.functions))
+            out["shaping"][name] = {"x": convert_x_matrix(x, d.nodes, d.functions), "c": convert_c_matrix(c, d.functions, d.nodes)}
+    for name, p, alpha in small_payloads():
+        a = arrays_of(p)
+        for kind in ("min_delay", "min_util", "min_delay_util"):
+            m = model.build_step1(a, kind, alpha)
+            out["model"][f"{name}|{kind}"] = model_digest(m["A"], m["lo"], m["hi"], m["obj"], m["lb"], m["ub"], m["integ"])
+            for strict in (True, False):
+                try:
+                    res = efttc.solve(a, kind, alpha, strict=strict)
+                except KeyError:
+                    rec = {"keyerror": True}
+                else:
+                    nz = np.flatnonzero(res.x)
+                    rec = {"keyerror": False, "c": res.c.astype(int).tolist(), "x_shape": list(res.x.shape),
+                           "x_index": nz.tolist(), "x_value": res.x.ravel()[nz].tolist(),
+                           "score": float(efttc.score(a, kind, alpha, res))}
+                out["efttc"][f"{name}|{kind}|{'strict' if strict else 'discard'}"] = rec
+    _dump("reference_vectors.json", out, indent=None)
+
+
 def make_lp_cut():
     """HiGHS optima of the slot-cut relaxation (oracle.relax) for the C2 seeds and a C5 subsample: pins the
     bound the matrix-free PDHG reports."""
@@ -297,7 +338,7 @@ if __name__ == "__main__":
     a = ap.parse_args()
     steps = {"alibaba": make_alibaba, "c1": make_c1, "payload_json": make_payload_json, "simulated": lambda: make_simulated(a.jobs),
              "model_hashes": make_model_hashes, "random_small": lambda: make_random_small(a.jobs),
-             "mip_optima": lambda: make_mip_optima(a.jobs), "lp_cut": make_lp_cut}
+             "mip_optima": lambda: make_mip_optima(a.jobs), "lp_cut": make_lp_cut, "reference_vectors": make_reference_vectors}
     for name, fn in steps.items():
         if a.only in (None, name):
             fn()

@@ -10,7 +10,6 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs the read-only reference tree at /root/reference")
 
 
 def pytest_collection_modifyitems(config, items):

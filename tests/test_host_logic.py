@@ -1,31 +1,13 @@
 """Host-side logic on CPU: the input adapter's defaults and edge cases, response shaping, error behaviour."""
-import contextlib
-import io
 import json
 
 import numpy as np
 import pytest
 
+from helpers import DATA_FIELDS, data_of, edge_payloads, reference_vectors, shaping_solution
 from neptune_mip_b200 import synth
 from neptune_mip_b200.core import check_input, data_to_solver_input
 from neptune_mip_b200.core.solvers.output import convert_c_matrix, convert_x_matrix
-from oracle.refshim import load_reference as L
-
-FIELDS = ["node_memory_matrix", "function_memory_matrix", "node_delay_matrix", "workload_matrix", "max_delay_matrix",
-          "node_cores_matrix", "cores_matrix", "old_allocations_matrix", "core_per_req_matrix", "node_costs"]
-
-
-def edge_payloads():
-    out = {"payload_json": synth.payload_json_sample()}
-    p = synth.test_py_payload(); p["workload_coeff"] = 2.5; out["workload_coeff"] = p
-    p = synth.random_payload(6, 3, 0, node_cores=10); p["actual_cpu_allocations"] = {"ns/fn_0": {}, "ns/fn_2": {"node_3": False}}
-    out["empty_and_false_allocations"] = p
-    p = synth.random_payload(5, 2, 1, node_cores=10)
-    p["workload_on_destination_matrix"] = [[0, 1, 0, 2, 0], [0, 0, 0, 0, 0]]      # x/0 -> DBL_MAX, 0/0 -> 0
-    p["cores_matrix"] = [[0, 1, 3, 2, 0], [0, 0, 0, 0, 1]]
-    out["division_by_zero"] = p
-    p = synth.simulated_case(0); out["one_by_one"] = p
-    return out
 
 
 def test_defaults_without_reference():
@@ -70,26 +52,16 @@ def test_response_shaping():
         convert_x_matrix(x[:1], nodes, funcs)
 
 
-@pytest.mark.skipif(not L.reference_available(), reason="reference tree not mounted")
 @pytest.mark.parametrize("name", list(edge_payloads()))
 def test_adapter_and_shaping_equal_the_reference_on_edge_cases(name):
-    core = L.load_reference()
+    """the reference's Data arrays and its convert_* responses on a random solution (golden/reference_vectors.json)"""
     payload = edge_payloads()[name]
-    coeff = payload.get("workload_coeff", 1)
-    with contextlib.redirect_stdout(io.StringIO()), np.errstate(all="ignore"):
-        core.check_input(payload)
-        rd = core.data_to_solver_input(payload, with_db=False, workload_coeff=coeff)
+    rd, shaped = reference_vectors()["data"][name], reference_vectors()["shaping"][name]
     check_input(payload)
-    md = data_to_solver_input(payload, coeff, with_db=False)
-    for k in FIELDS:
-        assert np.array_equal(np.asarray(getattr(rd, k)), np.asarray(getattr(md, k))), k
-    assert rd.nodes == md.nodes and rd.functions == md.functions and rd.node_budget == md.node_budget
-    # response shaping against the reference's own convert_* on a random solution
-    import sys
-    ref_out = sys.modules["core.solvers.neptune.utils.output"]
-    rng = np.random.default_rng(0)
-    N, F = len(md.nodes), len(md.functions)
-    x = rng.random((N, F, N)) * (rng.random((N, F, N)) < 0.3)
-    c = (rng.random((F, N)) < 0.4).astype(float)
-    assert convert_x_matrix(x, md.nodes, md.functions) == ref_out.convert_x_matrix(x, md.nodes, md.functions)
-    assert convert_c_matrix(c, md.functions, md.nodes) == ref_out.convert_c_matrix(c, md.functions, md.nodes)
+    md = data_of(payload)
+    for k in DATA_FIELDS:
+        assert np.array_equal(np.asarray(rd[k]), np.asarray(getattr(md, k))), k
+    assert rd["nodes"] == md.nodes and rd["functions"] == md.functions and rd["node_budget"] == md.node_budget
+    x, c = shaping_solution(len(md.nodes), len(md.functions))
+    assert convert_x_matrix(x, md.nodes, md.functions) == shaped["x"]
+    assert convert_c_matrix(c, md.functions, md.nodes) == shaped["c"]

@@ -1,91 +1,48 @@
-"""Oracle vs the UNMODIFIED reference code (imported read-only through oracle.refshim).
-Skipped where /root/reference does not exist (the GPU box)."""
-import contextlib
-import io
-import sys
-
+"""Input adapter and oracle vs what the UNMODIFIED reference computes on the payloads of helpers.py: its Data arrays, the
+digests of the step-1 matrices its builders emit, its EFTTC x, c, score and KeyError behaviour.  The reference's values are
+stored in golden/reference_vectors.json (oracle/make_golden.py: make_reference_vectors)."""
 import numpy as np
 import pytest
 
-from helpers import data_of, small_payloads
+from helpers import DATA_FIELDS, arrays_of, data_of, reference_vectors, small_payloads
 from oracle import efttc as oefttc, model as omodel
-from oracle.refshim import load_reference as L
+from oracle.make_golden import model_digest
 
-pytestmark = pytest.mark.skipif(not L.reference_available(), reason="reference tree not mounted")
-
-STEP1 = {"min_delay": "NeptuneStep1CPUMinDelay", "min_util": "NeptuneStep1CPUMinUtilization",
-         "min_delay_util": "NeptuneStep1CPUMinDelayAndUtilization"}
-EFTTC = {"min_delay": "EfttcStep1CPUMinDelay", "min_util": "EfttcStep1CPUMinUtilization",
-         "min_delay_util": "EfttcStep1CPUMinDelayAndUtilization"}
-
-
-def _ref_data(core, payload):
-    with contextlib.redirect_stdout(io.StringIO()), np.errstate(all="ignore"):
-        return core.data_to_solver_input(payload, with_db=False, workload_coeff=payload.get("workload_coeff", 1))
+KINDS = ["min_delay", "min_util", "min_delay_util"]
 
 
 @pytest.mark.parametrize("name,payload,alpha", small_payloads(), ids=lambda v: v if isinstance(v, str) else None)
 def test_input_adapter_equals_reference(name, payload, alpha):
-    core = L.load_reference()
-    rd, md = _ref_data(core, payload), data_of(payload)
-    for k in ["node_memory_matrix", "function_memory_matrix", "node_delay_matrix", "workload_matrix",
-              "max_delay_matrix", "node_cores_matrix", "cores_matrix", "old_allocations_matrix",
-              "core_per_req_matrix", "node_costs"]:
-        assert np.array_equal(np.asarray(getattr(rd, k)), np.asarray(getattr(md, k))), k
-    assert rd.node_budget == md.node_budget and rd.nodes == md.nodes and rd.functions == md.functions
+    want, md = reference_vectors()["data"][name], data_of(payload)
+    for k in DATA_FIELDS:
+        assert np.array_equal(np.asarray(want[k]), np.asarray(getattr(md, k))), k
+    assert want["node_budget"] == md.node_budget and want["nodes"] == md.nodes and want["functions"] == md.functions
 
 
 @pytest.mark.parametrize("name,payload,alpha", small_payloads(), ids=lambda v: v if isinstance(v, str) else None)
-@pytest.mark.parametrize("kind", list(STEP1))
+@pytest.mark.parametrize("kind", KINDS)
 def test_model_equals_reference_built_matrix(name, payload, alpha, kind):
-    core = L.load_reference()
-    solvers = sys.modules["core.solvers"]
-    data = _ref_data(core, payload)
-    with contextlib.redirect_stdout(io.StringIO()):
-        kw = dict(verbose=False)
-        if kind == "min_delay_util":
-            kw["alpha"] = alpha
-        s = getattr(solvers, STEP1[kind])(**kw)
-        s.load_data(data)
-        s.init_objective()
-    A, lo, hi, obj, lb, ub, integ = s.solver.export()
-    m = omodel.build_step1(omodel.arrays_from_data(data), kind, alpha)
-    assert np.array_equal(A.indptr, m["A"].indptr) and np.array_equal(A.indices, m["A"].indices)
-    assert np.array_equal(A.data, m["A"].data)
-    for k, v in dict(lo=lo, hi=hi, obj=obj, lb=lb, ub=ub, integ=integ).items():
-        assert np.array_equal(v, m[k]), k
+    want = reference_vectors()["model"][f"{name}|{kind}"]
+    m = omodel.build_step1(arrays_of(payload), kind, alpha)
+    got = model_digest(m["A"], m["lo"], m["hi"], m["obj"], m["lb"], m["ub"], m["integ"])
+    for k in ("shape", "nnz", "pattern", "data", "rows", "cols"):
+        assert got[k] == want[k], k
 
 
 @pytest.mark.parametrize("name,payload,alpha", small_payloads(), ids=lambda v: v if isinstance(v, str) else None)
-@pytest.mark.parametrize("kind", list(EFTTC))
+@pytest.mark.parametrize("kind", KINDS)
 @pytest.mark.parametrize("strict", [True, False])
 def test_efttc_equals_reference(name, payload, alpha, kind, strict):
-    core = L.load_reference()
-    solvers = sys.modules["core.solvers"]
-    L.enable_efttc_discard_patch(not strict)
-    try:
-        ref_err = None
-        with contextlib.redirect_stdout(io.StringIO()):
-            data = _ref_data(core, payload)
-            kw = dict(verbose=False)
-            if kind == "min_delay_util":
-                kw["alpha"] = alpha
-            s = getattr(solvers, EFTTC[kind])(**kw)
-            s.load_data(data)
-            try:
-                s.solve()
-                rx, rc = s.results()
-                rs = s.score()
-            except KeyError as e:
-                ref_err = e
-    finally:
-        L.enable_efttc_discard_patch(False)
-    a = omodel.arrays_from_data(data)
-    if ref_err is not None:
+    """strict: the reference as shipped; otherwise with `remaining_functions.remove` behaving like `discard`"""
+    want = reference_vectors()["efttc"][f"{name}|{kind}|{'strict' if strict else 'discard'}"]
+    a = arrays_of(payload)
+    if want["keyerror"]:
         with pytest.raises(KeyError):
             oefttc.solve(a, kind, alpha, strict=strict)
         return
     res = oefttc.solve(a, kind, alpha, strict=strict)
-    assert np.array_equal(rc, res.c) and np.array_equal(rx, res.x)
+    x = np.zeros(want["x_shape"])
+    x.ravel()[want["x_index"]] = want["x_value"]
+    assert np.array_equal(np.array(want["c"]), res.c) and np.array_equal(x, res.x)
     got = oefttc.score(a, kind, alpha, res)
-    assert got == rs or np.isclose(got, rs, rtol=1e-15, atol=0)
+    assert got == want["score"] or np.isclose(got, want["score"], rtol=1e-15, atol=0)
