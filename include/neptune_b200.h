@@ -178,10 +178,12 @@ int neptune_pdhg_mf_solve_util(int B, int N, int F, int kind, const double* d_ob
                                neptune_pdhg_result* result_d, void* workspace, int64_t workspace_bytes,
                                void* stream);
 
-/* ---- (b, matrix-free, sharded) EXPERIMENTAL: step-wise building blocks of the matrix-free iteration for the
- * function-block-sharded solver (neptune_mip_b200/sharded_mf.py, one process per GPU; SURVEY.md section 8(e)).  Not yet
- * run on a GPU (written after round 1's GPU budget was spent); the numpy statement they follow is
- * tests/mf_reference.ShardedMatrixFree.  F = functions of THIS rank; x / y / xsum / ysum are the canonical vectors of
+/* ---- (b, matrix-free, sharded) step-wise building blocks of the matrix-free iteration for the
+ * function-block-sharded solver (neptune_mip_b200/sharded_mf.py, one process per GPU; SURVEY.md section 8(e)): a rank
+ * owns the functions of its block, the 2N coupling rows (C2 memory, C4 CPU) are replicated, and the caller all-reduces
+ * their activities once per iteration; step sizes are host scalars.  The numpy statement they follow is
+ * tests/mf_reference.ShardedMatrixFree; on B200 two NCCL ranks reproduce the single-rank iterates to 3e-17
+ * (profiles/r02_sharded_mf.md).  F = functions of THIS rank; x / y / xsum / ysum are the canonical vectors of
  * the rank's local model; S4[B][N], S2[B] are the GLOBAL Pock-Chambolle row scalings (caller all-reduces the sums);
  * coupling[B][2N] = [C4 activity of the pending pass | C2 activity of the new cbar] over the own functions.
  *   column_sums : once before the first local step (and after y was replaced): column sums of yS
@@ -202,33 +204,6 @@ int neptune_pdhg_mf_pass(int B, int N, int F, const double* d, const double* w, 
                          int have_pass, int run_pass, double* x, double* y, double* xsum, double* ysum,
                          const double* S4, const double* S2, void* workspace, int64_t workspace_bytes,
                          const double* coupling_sum, void* stream);
-
-/* ---- (b') step-wise PDHG building blocks for the function-block-sharded solver (one process per GPU,
- * SURVEY.md section 8(e)): GPU g owns the functions of its block, i.e. the x / c columns and the C1 / C3
- * rows of those functions; the coupling rows (C2 memory, C4 CPU) are replicated, every GPU computes
- * their partial activity over its own columns, the caller all-reduces (NCCL) and applies the update.
- * Step sizes are host scalars.  `plan` / `meta_h` come from neptune_spmv_plan (pattern analysed once). */
-int neptune_spmv_plan_bytes(int64_t n_rows, int64_t* bytes);
-int neptune_spmv_plan(int64_t n_rows, const int64_t* ptr, void* plan, int32_t* meta_h, void* stream);
-int neptune_pdhg_primal_step(int B, int64_t rows, int64_t cols, int64_t nnz, const int64_t* rowT_ptr,
-                             const int32_t* colT_idx, const double* valT, void* planT, const int32_t* metaT_h,
-                             const double* obj, const double* col_lb, const double* col_ub, const double* T,
-                             double tau, const double* y, double* x, double* xbar, double* xsum, void* stream);
-/* rows in [d0,d1) and [d2,d3) are deferred: their activity (A xbar)[r] is written to
- * act[B][(d1-d0)+(d3-d2)] instead of being applied */
-int neptune_pdhg_dual_step(int B, int64_t rows, int64_t cols, int64_t nnz, const int64_t* row_ptr,
-                           const int32_t* col_idx, const double* val, void* plan, const int32_t* meta_h,
-                           const double* lo, const double* hi, const double* S, double sigma, const double* xbar,
-                           double* y, double* ysum, int64_t d0, int64_t d1, int64_t d2, int64_t d3, double* act,
-                           void* stream);
-int neptune_pdhg_dual_rows(int B, int64_t rows, int64_t d0, int64_t d1, int64_t d2, int64_t d3, double sigma,
-                           const double* act, const double* lo, const double* hi, const double* S, double* y,
-                           double* ysum, void* stream);
-/* |A| column sums / row sums (use_sum=1) or maxima (use_sum=0) under the scalings dr, dc; rowacc is
- * accumulated with atomics (zero it first); free rows (-inf,+inf) are ignored */
-int neptune_abs_sums(int B, int64_t rows, int64_t cols, int64_t nnz, const int64_t* rowT_ptr,
-                     const int32_t* colT_idx, const double* valT, const double* lo, const double* hi,
-                     const double* dr, const double* dc, int use_sum, double* colacc, double* rowacc, void* stream);
 
 /* ---- (c) exact evaluation, rounding, local search -------------------------------------------------
  * neptune_check_solution: the reference's six checkers and three scorers

@@ -50,14 +50,6 @@ _SIGNATURES = {
     "neptune_pdhg_mf_column_sums": [_i, _i, _i] + [_p] * 9 + [_p, _i64, _p],
     "neptune_pdhg_mf_local_step": [_i, _i, _i] + [_p] * 3 + [_d, _d, _i, _i] + [_p] * 6 + [_p, _i64, _p, _p],
     "neptune_pdhg_mf_pass": [_i, _i, _i] + [_p] * 6 + [_d, _d, _d, _i, _i] + [_p] * 6 + [_p, _i64, _p, _p],
-    "neptune_spmv_plan_bytes": [_i64, C.POINTER(_i64)],
-    "neptune_spmv_plan": [_i64, _p, _p, C.POINTER(C.c_int32), _p],
-    "neptune_pdhg_primal_step": [_i, _i64, _i64, _i64, _p, _p, _p, _p, C.POINTER(C.c_int32), _p, _p, _p, _p, _d,
-                                 _p, _p, _p, _p, _p],
-    "neptune_pdhg_dual_step": [_i, _i64, _i64, _i64, _p, _p, _p, _p, C.POINTER(C.c_int32), _p, _p, _p, _d, _p,
-                               _p, _p, _i64, _i64, _i64, _i64, _p, _p],
-    "neptune_pdhg_dual_rows": [_i, _i64, _i64, _i64, _i64, _i64, _d, _p, _p, _p, _p, _p, _p, _p],
-    "neptune_abs_sums": [_i, _i64, _i64, _i64, _p, _p, _p, _p, _p, _p, _p, _i, _p, _p, _p],
     "neptune_spmv": [_i, _i64, _i64, _p, _p, _p, _p, _p, _p],
     "neptune_spmv_t": [_i, _i64, _i64, _p, _p, _p, _p, _p, _p],
     "neptune_check_solution": [_i, _i, _i, _d] + _INST + [_p] * 5 + [_p],

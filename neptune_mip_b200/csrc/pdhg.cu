@@ -738,163 +738,3 @@ extern "C" int neptune_pdhg_solve(int B, int64_t rows, int64_t cols, int64_t nnz
   cudaStreamDestroy(s);
   return 0;
 }
-
-// ===================================================================================================
-// Step-wise building blocks for the function-block-sharded PDHG (SURVEY.md section 8(e)): the caller
-// (neptune_mip_b200/sharded.py, one process per GPU) owns the loop and the NCCL all-reduce of the
-// coupling rows; step sizes are host scalars, so no control block is needed.
-// ===================================================================================================
-namespace neptune {
-
-struct PrimalStep {          // x+ = clip(x - tau*T*(obj + A^T y)); xbar = 2x+ - x; xsum += x+
-  typedef PrimalUpdate::Pre Pre;
-  double tau; int64_t cols;
-  const double *obj, *lb, *ub, *T;
-  double *x, *xbar, *xsum;
-  __device__ bool skip(int) const { return false; }
-  __device__ double xscale(int) const { return 1.0; }
-  __device__ Pre pre(int b, int64_t c) const {
-    const int64_t k = (int64_t)b * cols + c;
-    return Pre{x[k], obj[k], T[k], lb[k], ub[k], xsum[k]};
-  }
-  __device__ void row(int b, int64_t c, double g, const Pre& p) const {
-    const int64_t k = (int64_t)b * cols + c;
-    double xn = p.xo - tau * p.t * (p.o + g);
-    xn = fmin(fmax(xn, p.l), p.u);
-    x[k] = xn; xbar[k] = 2.0 * xn - p.xo; xsum[k] = p.s + xn;
-  }
-  __device__ void finalize(int) const {}
-};
-
-struct DualStep {            // dual update, except rows in [d0,d1) u [d2,d3): their activity goes to act[]
-  typedef DualUpdate::Pre Pre;
-  double sigma; int64_t rows;
-  const double *lo, *hi, *S;
-  double *y, *ysum;
-  int64_t d0, d1, d2, d3;
-  double* act;
-  __device__ bool skip(int) const { return false; }
-  __device__ double xscale(int) const { return 1.0; }
-  __device__ Pre pre(int b, int64_t r) const {
-    const int64_t k = (int64_t)b * rows + r;
-    return Pre{y[k], S[k], lo[k], hi[k], ysum[k]};
-  }
-  __device__ void row(int b, int64_t r, double a, const Pre& p) const {
-    const int64_t nd = (d1 - d0) + (d3 - d2);
-    if (r >= d0 && r < d1) { act[(int64_t)b * nd + (r - d0)] = a; return; }
-    if (r >= d2 && r < d3) { act[(int64_t)b * nd + (d1 - d0) + (r - d2)] = a; return; }
-    const int64_t k = (int64_t)b * rows + r;
-    const double s = sigma * p.sc;
-    const double v = p.yo + s * a;
-    const double yn = (isinf(p.l) && isinf(p.h)) ? 0.0 : v - s * fmin(fmax(v / s, p.l), p.h);   // free row: exactly 0
-    y[k] = yn; ysum[k] = p.s + yn;
-  }
-  __device__ void finalize(int) const {}
-};
-
-// dual update of the deferred rows from their (all-reduced) activities
-__global__ void k_dual_rows(int64_t n0, int64_t n1, int64_t d0, int64_t d2, int64_t rows, double sigma,
-                            const double* __restrict__ act, const double* __restrict__ lo,
-                            const double* __restrict__ hi, const double* __restrict__ S,
-                            double* __restrict__ y, double* __restrict__ ysum) {
-  const int b = blockIdx.y;
-  const int64_t nd = n0 + n1;
-  for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < nd; k += (int64_t)gridDim.x * blockDim.x) {
-    const int64_t r = (k < n0) ? d0 + k : d2 + (k - n0);
-    const int64_t q = (int64_t)b * rows + r;
-    const double s = sigma * S[q];
-    const double v = y[q] + s * act[(int64_t)b * nd + k];
-    const double yn = v - s * fmin(fmax(v / s, lo[q]), hi[q]);
-    y[q] = yn; ysum[q] += yn;
-  }
-}
-
-}  // namespace neptune
-
-extern "C" int neptune_spmv_plan_bytes(int64_t n_rows, int64_t* bytes) {
-  if (n_rows <= 0 || !bytes) return NEPTUNE_E_ARG;
-  *bytes = (int64_t)side_scratch_bytes(n_rows);
-  return 0;
-}
-
-// Analyse the pattern of one CSR matrix once (warp tasks, long rows); `plan` is device scratch of
-// neptune_spmv_plan_bytes(n_rows) bytes that the step functions below take back.  meta_h[3] (host):
-// {#long rows, has thread-per-row tasks, has warp tasks}.
-extern "C" int neptune_spmv_plan(int64_t n_rows, const int64_t* ptr, void* plan, int32_t* meta_h, void* stream) {
-  if (n_rows <= 0 || !ptr || !plan || !meta_h) return NEPTUNE_E_ARG;
-  Side S{};
-  S.M.ptr = ptr; S.M.n_rows = n_rows;
-  int rc = analyse_side(S, (char*)plan, (cudaStream_t)stream);
-  if (rc) return rc;
-  meta_h[0] = S.n_long_h; meta_h[1] = S.has_short; meta_h[2] = S.has_wide;
-  return 0;
-}
-
-static Side side_from_plan(const Csr& M, void* plan, const int32_t* meta_h) {
-  Side S{};
-  S.M = M;
-  char* mem = (char*)plan;
-  S.tasks = (int32_t*)mem; mem += (((size_t)(M.n_rows + 2) * 4 + 255) & ~(size_t)255);
-  S.long_rows = (int32_t*)mem; mem += (size_t)kMaxLongList * 4;
-  S.n_tasks = (int32_t*)mem; S.n_long = S.n_tasks + 1;
-  S.n_long_h = meta_h[0]; S.has_short = meta_h[1]; S.has_wide = meta_h[2];
-  return S;
-}
-
-extern "C" int neptune_pdhg_primal_step(int B, int64_t rows, int64_t cols, int64_t nnz, const int64_t* rowT_ptr,
-                                        const int32_t* colT_idx, const double* valT, void* planT,
-                                        const int32_t* metaT_h, const double* obj, const double* col_lb,
-                                        const double* col_ub, const double* T, double tau, const double* y,
-                                        double* x, double* xbar, double* xsum, void* stream) {
-  if (B <= 0 || !rowT_ptr || !colT_idx || !valT || !planT || !metaT_h || !obj || !col_lb || !col_ub || !T || !y ||
-      !x || !xbar || !xsum)
-    return NEPTUNE_E_ARG;
-  Plan P{};
-  P.B = B; P.rows = rows; P.cols = cols; P.nnz = nnz; P.s = (cudaStream_t)stream;
-  P.At = side_from_plan(Csr{rowT_ptr, colT_idx, valT, cols, rows, nnz}, planT, metaT_h);
-  launch_cols(P, y, PrimalStep{tau, cols, obj, col_lb, col_ub, T, x, xbar, xsum});
-  NEPTUNE_LAUNCH_OK();
-  return 0;
-}
-
-extern "C" int neptune_pdhg_dual_step(int B, int64_t rows, int64_t cols, int64_t nnz, const int64_t* row_ptr,
-                                      const int32_t* col_idx, const double* val, void* plan, const int32_t* meta_h,
-                                      const double* lo, const double* hi, const double* S, double sigma,
-                                      const double* xbar, double* y, double* ysum, int64_t d0, int64_t d1,
-                                      int64_t d2, int64_t d3, double* act, void* stream) {
-  if (B <= 0 || !row_ptr || !col_idx || !val || !plan || !meta_h || !lo || !hi || !S || !xbar || !y || !ysum)
-    return NEPTUNE_E_ARG;
-  if (d0 > d1 || d2 > d3 || ((d1 - d0) + (d3 - d2) > 0 && !act)) return NEPTUNE_E_ARG;
-  Plan P{};
-  P.B = B; P.rows = rows; P.cols = cols; P.nnz = nnz; P.s = (cudaStream_t)stream;
-  P.A = side_from_plan(Csr{row_ptr, col_idx, val, rows, cols, nnz}, plan, meta_h);
-  launch_rows(P, xbar, DualStep{sigma, rows, lo, hi, S, y, ysum, d0, d1, d2, d3, act});
-  NEPTUNE_LAUNCH_OK();
-  return 0;
-}
-
-extern "C" int neptune_pdhg_dual_rows(int B, int64_t rows, int64_t d0, int64_t d1, int64_t d2, int64_t d3,
-                                      double sigma, const double* act, const double* lo, const double* hi,
-                                      const double* S, double* y, double* ysum, void* stream) {
-  if (B <= 0 || d0 > d1 || d2 > d3 || !act || !lo || !hi || !S || !y || !ysum) return NEPTUNE_E_ARG;
-  const int64_t nd = (d1 - d0) + (d3 - d2);
-  if (nd == 0) return 0;
-  { k_dual_rows<<<dim3(grid1(nd, 256, 4), B), 256, 0, (cudaStream_t)stream>>>(d1 - d0, d3 - d2, d0, d2, rows, sigma,
-                                                                            act, lo, hi, S, y, ysum); NEPTUNE_COUNT(1); }
-  NEPTUNE_LAUNCH_OK();
-  return 0;
-}
-
-// |A| column sums (colacc[B][cols]) and row sums (rowacc[B][rows], accumulated with atomics: zero it
-// first) -- the Pock-Chambolle preconditioner T = 1/colsum, S = 1/rowsum of the sharded solver.
-extern "C" int neptune_abs_sums(int B, int64_t rows, int64_t cols, int64_t nnz, const int64_t* rowT_ptr,
-                                const int32_t* colT_idx, const double* valT, const double* lo, const double* hi,
-                                const double* dr, const double* dc, int use_sum, double* colacc, double* rowacc,
-                                void* stream) {
-  if (B <= 0 || !rowT_ptr || !colT_idx || !valT || !lo || !hi || !dr || !dc || !colacc || !rowacc) return NEPTUNE_E_ARG;
-  Csr At{rowT_ptr, colT_idx, valT, cols, rows, nnz};
-  dim3 g(grid1(cols, 256, 16), B);
-  { k_scale_pass<<<g, 256, 0, (cudaStream_t)stream>>>(At, use_sum, dr, dc, lo, hi, colacc, rowacc); NEPTUNE_COUNT(1); }
-  NEPTUNE_LAUNCH_OK();
-  return 0;
-}

@@ -1,4 +1,4 @@
-"""Function-block-sharded PDHG: 2 ranks must reproduce the unsharded iterates (one GPU, gloo for the
+"""Function-block-sharded matrix-free PDHG: 2 ranks must reproduce the unsharded iterates (one GPU, gloo for the
 exchange -- the NCCL path is the same code with `dist.all_reduce` on device tensors)."""
 import os
 import subprocess
@@ -8,27 +8,6 @@ import pytest
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-def test_two_ranks_match_single_rank():
-    env = dict(os.environ, NEPTUNE_DIST_BACKEND="gloo")
-    cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr",
-           "127.0.0.1", "--master-port", "29533", os.path.join(ROOT, "tools", "sharded_run.py"), "parity", "24", "6", "150"]
-    out = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
-    assert "PARITY world=2" in out.stdout
-
-
-def test_sharded_restarted_solve_reaches_the_single_gpu_lp_optimum():
-    """CPU-binding instance (non-zero LP optimum): two ranks, restarts decided from all-reduced KKT pieces."""
-    env = dict(os.environ, NEPTUNE_DIST_BACKEND="gloo", NEPTUNE_NODE_CORES="12")
-    cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr",
-           "127.0.0.1", "--master-port", "29534", os.path.join(ROOT, "tools", "sharded_run.py"), "solve", "8", "4", "40000"]
-    out = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=900)
-    assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
-    assert "SOLVE world=2" in out.stdout
-
-
 
 
 def test_matrix_free_single_rank_equals_the_numpy_iteration():
