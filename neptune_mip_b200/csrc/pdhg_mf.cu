@@ -24,7 +24,12 @@
 //   = 64*X, + 112*F*N (small vectors) + 8*N*N (d, re-read per function from L1/L2)  [X = F*N*N]; the CSR solver
 //   moves 16*nnz + 88*cols + 72*rows ~ 260*X for the same iteration.
 //
-// Three iteration passes, all parity-tested against the numpy statement (tests/test_pdhg_mf_gpu.py):
+// Three iteration passes, all parity-tested against the numpy statement: tests/test_pdhg_mf_gpu.py up to 70 x 3 and
+// 50 x 10; tests/test_pdhg_mf_wide_gpu.py at the branches only wide shapes take, each case pinned to its branch by
+// neptune_pdhg_mf_geometry -- k_mf_iter<4, U> / k_mf_eval<4> (65 x 8, 99 x 5, 129 x 40), the C4 dual in 16 slices
+// (K4 = F * rt from 65 to 800, the C3 bench instance included), k_mf_small on many blocks with the C2 dual in its own
+// launch (F * N > 4096: 130 x 33, 129 x 40, C3, the node-column models), the bulk-copy pass with 64 and 80 functions,
+// 17 column tiles (1026 x 2) -- and the restarted solve, decision by decision, against mf_reference.solve_ctl:
 //   k_mf_iter_bulk<RED, FUSE> (pdhg_mf_bulk.cuh; even N <= 64, the default for even N in 34..64, i.e. C2): the streams
 //     staged through shared memory by the bulk-copy engine (cp.async.bulk + mbarrier), running sums by
 //     cp.reduce.async.bulk add.f64, the small-vector update inside the same launch -- 0.75-0.79 of the measured HBM peak
@@ -1080,7 +1085,8 @@ using namespace neptune;
 
 // host-only: the tile geometry the solver would use (tests, tools).  out[0..7] = {K columns per lane, JT columns per
 // tile, ct column tiles, RT rows per tile, rt row tiles, tiles per instance, F*N <= 4096 (single-block small
-// kernel), 0}; out[8..15] = geometry of the bulk-copy pass (below)
+// kernel), the default bulk-copy pass of a min-delay solve with an even graph replay runs the small-vector update
+// inside its launches}; out[8..15] = geometry of the bulk-copy pass (below)
 extern "C" int neptune_pdhg_mf_geometry(int B, int N, int F, int32_t* out) {
   if (B <= 0 || N <= 0 || F <= 0 || !out) return NEPTUNE_E_ARG;
   const MfGeo G = make_geo(N, F, B);
@@ -1096,6 +1102,7 @@ extern "C" int neptune_pdhg_mf_geometry(int B, int N, int F, int32_t* out) {
     out[11] = c2.ok; out[12] = c2.stages; out[13] = c2.nw; out[15] = (int32_t)c2.smem;
     const int dflt = N > 32 ? mf_default_bulk() : 0;
     out[14] = (dflt == 1 && c4.ok) ? 1 : ((dflt == 2 && c2.ok) ? 2 : 0);
+    out[7] = out[14] ? bulk_config(N, out[14] == 2, 0, 0, F, 1).ok : 0;     // as mf_choose_pass: the fused config fits
   }
   return 0;
 }

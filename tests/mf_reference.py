@@ -363,6 +363,95 @@ def solve(mf: MatrixFree, max_iters=20000, check=64, eps=1e-6, verbose=False):
     return dict(primal=cands[pick][4], dual=cands[pick][5], iters=it, restarts=restarts, converged=False)
 
 
+def solve_ctl(mf: MatrixFree, max_iters, check_every, eps_abs, eps_rel):
+    """The restarted solve exactly as `neptune_pdhg_mf_solve` takes it: chunks of `check_every` iterations (the last
+    one cut at max_iters), then the decision of k_ctl_decide and the primal-weight update of k_ctl_after_restart.
+    Unlike `solve`, the final check (converged or out of iterations) takes no restart and leaves the better candidate
+    in the state, and the absolute and relative tolerances are separate.
+
+    Returns (info, log).  info: the device's result record (primal_obj, dual_obj, primal_res, dual_res,
+    primal_weight, iters, restarts, converged).  log: one dict per check with the KKT errors of both candidates, the
+    pick, the action (0 none, 1 restart to the average, 2 restart at the current iterate) and `decisions`, the
+    floating-point comparisons the device evaluated at that check as (label, value, threshold) -- in the order and
+    with the short-circuits of k_ctl_decide, so that a test can ask how far each was from going the other way."""
+    omega = mf.omega
+    sums = [np.zeros_like(t) for t in mf.state()]
+    rst = [np.array(t) for t in mf.state()]
+    iters = since = count = restarts = 0
+    kr = kp = np.inf
+    log = []
+    while True:
+        chunk = min(check_every, max_iters - iters)
+        for _ in range(chunk):
+            mf.step()
+            for s_, t in zip(sums, mf.state()):
+                s_ += t
+        iters += chunk; since += chunk; count += chunk
+        avg = tuple(s_ / count for s_ in sums)
+        decisions, kkt, ok, nums = [], [], [], []
+        for st in (mf.state(), avg):
+            p2, d2, po, do = mf.kkt(st)
+            gap = abs(po - do)
+            kkt.append(np.sqrt(omega * omega * p2 + d2 / (omega * omega) + gap * gap))
+            tests = [("primal residual", np.sqrt(p2), eps_abs + eps_rel * mf.nb),
+                     ("dual residual", np.sqrt(d2), eps_abs + eps_rel * mf.nc),
+                     ("gap", gap, eps_abs + eps_rel * (abs(po) + abs(do)))]
+            good = True
+            for t in tests:                                   # && of k_ctl_decide: stops at the first failure
+                decisions.append(t)
+                if not t[1] <= t[2]:
+                    good = False
+                    break
+            ok.append(good)
+            nums.append((po, do, np.sqrt(p2), np.sqrt(d2)))
+        if ok[0] == ok[1]:
+            decisions.append(("average vs current KKT", kkt[1], kkt[0]))
+            pick = 1 if kkt[1] < kkt[0] else 0
+        else:
+            pick = 1 if ok[1] else 0
+        done = ok[0] or ok[1]
+        last = done or iters >= max_iters
+        cand = kkt[pick]
+        action = 0
+        if not last:
+            decisions.append(("sufficient decay", cand, 0.2 * kr))
+            if cand <= 0.2 * kr:
+                action = 1 + (pick == 0)
+            else:
+                decisions.append(("necessary decay", cand, 0.8 * kr))
+                if cand <= 0.8 * kr:
+                    decisions.append(("no progress", cand, kp))
+                if cand <= 0.8 * kr and cand > kp:
+                    action = 1 + (pick == 0)
+                elif since >= 0.36 * iters and iters > 0 and restarts > 0:
+                    action = 1 + (pick == 0)
+                elif restarts == 0 and since >= 4 * chunk:
+                    action = 1 + (pick == 0)
+        kp = cand
+        if action:
+            kr = cand; restarts += 1
+        log.append(dict(iters=iters, kkt=tuple(kkt), ok=tuple(ok), pick=pick, action=action if not last else 0,
+                        decisions=decisions))
+        po, do, pres, dres = nums[pick]
+        info = dict(primal_obj=po, dual_obj=do, primal_res=pres, dual_res=dres, primal_weight=omega, iters=iters,
+                    restarts=restarts, converged=int(done))
+        if last:
+            if pick == 1:                                     # the average is materialised into x, y
+                mf.set_state(avg)
+            return info, log
+        if action:
+            if action == 1:
+                mf.set_state(avg)
+            st = mf.state()
+            dx, dy = mf.movement(st, rst)
+            if dx > 1e-10 and dy > 1e-10 and np.isfinite(dx) and np.isfinite(dy):
+                nw = np.exp(0.5 * np.log(dy / dx) + 0.5 * np.log(omega))
+                omega = min(max(nw, 0.5 * omega), 2.0 * omega)
+            mf.omega = omega                                  # MatrixFree.step takes tau, sigma from it
+            rst = [np.array(t) for t in st]
+            for s_ in sums:
+                s_[:] = 0
+            since = count = 0
 
 
 def run_fixed(a, iters, kind="min_delay", alpha=0.5, bigm=None):

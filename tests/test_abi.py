@@ -81,8 +81,12 @@ def test_matrix_free_tile_geometry_covers_every_shape():
             if ok4:
                 assert st4 >= 2 and st4 * (5 * slab + vec) <= 227 * 1024
         assert dflt in (0, 1, 2) and (N > 32 or dflt == 0)
+        assert out[7] in (0, 1) and (out[7] == 0 or dflt != 0)        # small-vector update inside the bulk pass
         assert lib.neptune_pdhg_mf_workspace_bytes(B, N, F, ctypes.byref(need)) == 0
         X, C = F * N * N, F * N
         assert need.value >= 8 * B * (2 * (X + C) + 2 * (3 * C + 2 * N + X))        # xsum, xres, ysum, yres at least
+    # C2 (50 x 10) runs the small-vector update inside the bulk pass; with 80 functions its two buffers do not fit
+    for (N, F, fused) in [(50, 10, 1), (50, 80, 0), (64, 3, 0), (34, 3, 1), (12, 5, 0)]:
+        assert lib.neptune_pdhg_mf_geometry(256, N, F, out) == 0 and out[7] == fused, (N, F)
     assert lib.neptune_pdhg_mf_geometry(0, 3, 2, out) == -1
     assert lib.neptune_pdhg_mf_workspace_bytes(1, 4000, 400, ctypes.byref(need)) == -2

@@ -11,13 +11,15 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def test_matrix_free_single_rank_equals_the_numpy_iteration():
-    """world size 1: the step-wise entry points (local step / pass / flush) reproduce tests/mf_reference.MatrixFree"""
+    """world size 1: the step-wise entry points (local step / pass / flush) reproduce tests/mf_reference.MatrixFree;
+    65 x 8 runs four strided columns per lane, 130 x 33 three column tiles and 17 row tiles (561 partial sums per column
+    of the C4 activity), both with CPU capacities tight enough that the C4 rows bind"""
     import numpy as np
     from helpers import arrays_of, data_of
     from mf_reference import MatrixFree
     from neptune_mip_b200 import synth
     from neptune_mip_b200.sharded_mf import ShardedMF
-    for (N, F, cores, iters) in ((12, 5, 25, 96), (50, 4, 200, 40), (70, 3, 60, 33)):
+    for (N, F, cores, iters) in ((12, 5, 25, 96), (50, 4, 200, 40), (70, 3, 60, 33), (65, 8, 38, 33), (130, 33, 154, 33)):
         p = synth.random_payload(N, F, 1, node_cores=cores)
         lp = ShardedMF(data_of(p))
         ref = MatrixFree(arrays_of(p))
@@ -41,6 +43,17 @@ def test_matrix_free_two_ranks_match_single_rank():
     out = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=600)
     assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
     assert "MF-PARITY world=2" in out.stdout
+
+
+def test_matrix_free_two_ranks_match_single_rank_uneven_split():
+    """33 functions over 2 ranks (17 + 16): the ranks' blocks differ in size, and 130 nodes give three column tiles and
+    many row tiles per function; tight CPU capacities make the replicated C4 dual move"""
+    env = dict(os.environ, NEPTUNE_DIST_BACKEND="gloo", NEPTUNE_NODE_CORES="154")
+    cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr",
+           "127.0.0.1", "--master-port", "29537", os.path.join(ROOT, "tools", "sharded_run.py"), "mf-parity", "130", "33", "70"]
+    out = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
+    assert "MF-PARITY world=2 N=130 F=33" in out.stdout
 
 
 def test_matrix_free_sharded_solve_reaches_the_single_gpu_optimum():
