@@ -255,6 +255,9 @@ int neptune_local_search(int B, int N, int F, int kind, double alpha, int chains
                          uint8_t* best_c, double* best_obj, int32_t* best_flags,
                          void* workspace, int64_t workspace_bytes, void* stream);
 int neptune_local_search_workspace_bytes(int B, int N, int F, int chains, int64_t* bytes);
+/* *fits = 1 when neptune_local_search (and neptune_disruption_search) take instances of N nodes and F functions,
+ * 0 when they return NEPTUNE_E_SIZE for them (a chain's shared-memory rows exceed 200 KiB: N > 1066).  Host only. */
+int neptune_local_search_fits(int N, int F, int32_t* fits);
 
 /* neptune_disruption_search: step 2 "minimise disruption" (reference NeptuneStep2*, neptune_step2.py:5-93,
  * constraints_step2.py:5-89, objectives.py:55-63) as a search over placements with the step-2 objective in
@@ -319,6 +322,20 @@ int neptune_lns_block_mode(int mode);
 int neptune_site_greedy_workspace_bytes(int B, int N, int F, int64_t* bytes);
 int neptune_site_greedy(int B, int N, int F, const double* d, const double* w, const double* m, const double* Mj,
                         double unserved_delay, int max_rounds, uint8_t* c_out, int32_t* info_out,
+                        void* workspace, int64_t workspace_bytes, void* stream);
+
+/* neptune_site_search: best-improvement pod-exchange search for the min-delay objective under nearest-pod routing,
+ * obj = sum_f sum_i w[f,i] * (delay from i to the nearest open pod of f), at any size (csrc/site_search.cu).  Starts
+ * from c_in[B][F][N] (uint8; every function with a pod, memory rows sum_f m[f] c[f,j] <= Mj held; e.g.
+ * neptune_site_greedy's placement) and keeps both.  Per round every node proposes its best add or exchange (one
+ * function leaves, another enters), every function its best relocation of one pod; proposals touching disjoint
+ * functions and nodes are accepted in order of improvement.  Stops when a round accepts nothing or after max_rounds.
+ * c_out[B][F][N] (may equal c_in), info_out[B][4] = {rounds that accepted a move, adds, exchanges, relocations},
+ * obj_out[B][2] = {objective at the start, at the end}.  Deterministic.  NEPTUNE_E_ARG when a function of c_in has
+ * no pod.  Workspace from neptune_site_search_workspace_bytes. */
+int neptune_site_search_workspace_bytes(int B, int N, int F, int64_t* bytes);
+int neptune_site_search(int B, int N, int F, const double* d, const double* w, const double* m, const double* Mj,
+                        const uint8_t* c_in, uint8_t* c_out, int max_rounds, int32_t* info_out, double* obj_out,
                         void* workspace, int64_t workspace_bytes, void* stream);
 
 /* neptune_route_two_choice: routing of ONE placement per instance at sizes where the per-instance routers do not

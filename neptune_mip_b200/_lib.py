@@ -59,6 +59,8 @@ _SIGNATURES = {
     "neptune_route_lp_workspace_bytes": [_i, _i, _i, _i, _i64, C.POINTER(_i64)],
     "neptune_site_greedy_workspace_bytes": [_i, _i, _i, C.POINTER(_i64)],
     "neptune_site_greedy": [_i, _i, _i, _p, _p, _p, _p, _d, _i, _p, _p, _p, _i64, _p],
+    "neptune_site_search_workspace_bytes": [_i, _i, _i, C.POINTER(_i64)],
+    "neptune_site_search": [_i, _i, _i, _p, _p, _p, _p, _p, _p, _i, _p, _p, _p, _i64, _p],
     "neptune_route_two_choice_workspace_bytes": [_i, _i, _i, C.POINTER(_i64)],
     "neptune_route_two_choice": [_i, _i, _i] + [_p] * 4 + [_p] * 6 + [C.POINTER(C.c_int32), _i, _p, _i64, _p],
     "neptune_lns_block_mode": [_i],
@@ -67,6 +69,7 @@ _SIGNATURES = {
     "neptune_local_search": [_i, _i, _i, _i, _d, _i, _i, C.c_uint64, _i] + _INST + [_p] * 6 + [_p, _i64, _p],
     "neptune_disruption_search": [_i, _i, _i, _i, _d, _i, _p, _i, _i, C.c_uint64, _i] + _INST + [_p] * 5 + [_p, _i64, _p],
     "neptune_local_search_workspace_bytes": [_i, _i, _i, _i, C.POINTER(_i64)],
+    "neptune_local_search_fits": [_i, _i, C.POINTER(C.c_int32)],
     "neptune_efttc": [_i, _i, _i, _i, _d] + [_p] * 8 + [_d] + [_p] * 3 + [_p, _i64, _p],
     "neptune_efttc_workspace_bytes": [_i, _i, _i, C.POINTER(_i64)],
     "neptune_u8_to_f64": [_i64, _p, _p, _p],

@@ -1,5 +1,6 @@
 """Batched solve path: B same-shaped instances through the LP relaxation (PDHG: matrix-free for the min-delay
-model, assembly + CSR otherwise) -> EFTTC -> local search -> exact check in one go (what bench.py times, and what a sweep like BASELINE.json's config 5 calls)."""
+model, assembly + CSR otherwise) -> EFTTC -> local search (or, for the min-delay model at sizes the searches with
+shared-memory chain state do not take, greedy -> pod-exchange search -> two-choice routing) -> exact check in one go (what bench.py times, and what a sweep like BASELINE.json's config 5 calls)."""
 from __future__ import annotations
 
 import os
@@ -12,7 +13,10 @@ import numpy as np
 import torch
 
 from . import device
-from ._lib import FLAG_STRENGTHEN, KINDS, OK_ALL
+from ._lib import FLAG_STRENGTHEN, KINDS, OK_ALL, OK_C_X, OK_CPU, OK_HANDLE, OK_MEMORY, OK_N_C
+
+# the checks of the min-delay model: it has no budget row (C6), so the budget flag does not make its answer infeasible
+MIN_DELAY_FLAGS = OK_HANDLE | OK_MEMORY | OK_CPU | OK_C_X | OK_N_C
 
 
 @dataclass
@@ -25,7 +29,9 @@ class BatchParams:
     chains: int = 16              # local-search chains per instance (add/drop/swap search)
     sweeps: int = 200
     rng_seed: int = 1
-    search: str = "auto"          # "auto": slot-count LNS (csrc/lns.cu) where it applies, else the add/drop/swap search; "local": always the latter
+    search: str = "auto"          # "auto": slot-count LNS (csrc/lns.cu) where it applies, else the add/drop/swap search, and for the
+                                  # min-delay model at sizes neither takes (N > 1066) the pod-exchange search; "local": always the
+                                  # add/drop/swap search; "site": always the pod-exchange search (min-delay only)
     lp_cut: bool = True           # relax with the Chvatal-Gomory rounding of the memory rows (one memory size per instance)
     lns_chains: int = 96          # warp-sized chains per instance
     lns_fill_waves: bool = False  # raise the chain count (at most 1.5x) until the blocks of the search fill whole waves of the GPU
@@ -58,7 +64,7 @@ class BatchResult:
     model_dims: tuple = (0, 0, 0)
     pdhg_bytes_per_iter: int = 0  # algorithmic bytes one PDHG iteration of the whole batch moves (DESIGN.md section 3b)
     pdhg_path: str = ""           # "matrix-free" | "csr"
-    search_path: str = ""         # "lns" | "local"
+    search_path: str = ""         # "lns" | "local" | "site"
     lns_round: Optional[torch.Tensor] = None     # [B] round at which the returned placement was recorded by its chain
     lns_ms: float = 0.0
     lns_diag: Optional[dict] = None              # elite_g[B,E] priced objective, elite_val[B,E] exact objective (inf: infeasible)
@@ -71,7 +77,12 @@ def solve_batch(inst: device.InstanceBatch, prm: BatchParams, time_pdhg: bool = 
     use_lns = prm.search == "auto" and device.lns_supported(inst, kind)
     if use_lns and KINDS.get(kind, kind) == 2 and not bool((objective_weights(inst, kind, prm.alpha)[0] > 0).all()):
         use_lns = False         # no workload: the combined objective has no delay term (objectives.py:34-35), nothing to price
-    inst_lp = device.slot_relaxation(inst) if (use_lns and prm.lp_cut) else inst
+    use_site = prm.search == "site" or (prm.search == "auto" and KINDS.get(kind, kind) == 0 and not use_lns
+                                        and not device.local_search_fits(inst.N, inst.F))
+    if use_site and KINDS.get(kind, kind) != 0:
+        raise ValueError("search='site' solves the min-delay model only")
+    cut = prm.lp_cut and (use_lns or (use_site and device.one_memory_size(inst)))
+    inst_lp = device.slot_relaxation(inst) if cut else inst
     if prm.lp_iters > 0:
         N, F, B = inst.N, inst.F, inst.B
         X = F * N * N
@@ -109,6 +120,9 @@ def solve_batch(inst: device.InstanceBatch, prm: BatchParams, time_pdhg: bool = 
         iters = int(lp_res["iters"].max())
         guide = xs[:, X:X + F * N].contiguous()
         del xs, ys
+    if use_site:
+        best_c, x, n, flags, scores = site_step1(inst, prm.alpha)
+        return BatchResult(best_c, x, n, flags, scores, lp_res, pdhg_ms, iters, dims, bytes_iter, path, "site")
     cache = {}
 
     def get_seeds():
@@ -152,6 +166,29 @@ def solve_batch(inst: device.InstanceBatch, prm: BatchParams, time_pdhg: bool = 
                 break
     return BatchResult(best_c, x, n, flags, scores, lp_res, pdhg_ms, iters, dims, bytes_iter, path,
                        "lns" if use_lns else "local", lns_round, lns_ms, lns_diag)
+
+
+def site_step1(inst: device.InstanceBatch, alpha=0.5):
+    """Min-delay placement at any size: round-robin greedy -> pod-exchange search -> two-choice routing -> checkers.
+    The searched placement is kept where it passes the model's checks (MIN_DELAY_FLAGS) and routes no worse than the
+    greedy's; elsewhere the greedy's routed placement stands in.  Neither EFTTC nor the capacity-aware router runs here
+    (neither finishes at BASELINE config 4).  Returns (c uint8[B,F,N], x, n, flags, scores)."""
+    M = MIN_DELAY_FLAGS
+    cg, _ = device.site_greedy(inst)
+    cs, _, _ = device.site_search(inst, cg)
+    c, x, n, obj, _, _ = device.route_two_choice(inst, cs)
+    flags, scores = device.check_solution(inst, x, device.u8_to_f64(c), n, alpha)
+    _, _, _, obj_g, _, _ = device.route_two_choice(inst, cg, want_x=False)
+    failed = (flags & M) != M
+    bad = failed | (obj_g < obj)
+    if bool(bad.any()):
+        cf, xf, nf, _, _, _ = device.route_two_choice(inst, cg)
+        ff, sf = device.check_solution(inst, xf, device.u8_to_f64(cf), nf, alpha)
+        take = bad & (((ff & M) == M) | failed)
+        if bool(take.any()):
+            c[take], x[take], n[take], flags[take], scores[take] = cf[take], xf[take], nf[take], ff[take], sf[take]
+        del xf
+    return c, x, n, flags, scores
 
 
 _DEBUG_SYNC = int(os.environ.get("NEPTUNE_DEBUG_SYNC", "0"))

@@ -54,7 +54,9 @@ class NeptuneStepBase(GpuStepMixin, Solver):
 class NeptuneStep1CPUBase(NeptuneStepBase):
     def solve(self):
         """LP relaxation (bound, rounding guide, CPU-row prices) -> search -> exact routing LP -> the reference's
-        checkers, all through `batch.solve_batch` (the path bench.py times) with a batch of one."""
+        checkers, all through `batch.solve_batch` (the path bench.py times) with a batch of one.  Min-delay instances too
+        large for the searches with shared-memory chain state (N > 1066, BASELINE config 4) take the greedy ->
+        pod-exchange search -> two-choice routing path instead."""
         from ....batch import BatchParams, solve_batch
         self.init_objective()
         prm = BatchParams(kind=self.kind, alpha=self._alpha(), lp_iters=self.lp_iters, lp_check_every=256,

@@ -743,6 +743,11 @@ extern "C" int neptune_local_search_workspace_bytes(int B, int N, int F, int cha
   return 0;
 }
 
+// one row of N doubles per warp in shared memory; the only part of it that grows with N without bound
+static inline int ls_threads(int N) { return N > 128 ? 768 : 256; }
+static inline size_t ls_row_bytes(int N) { return (size_t)(ls_threads(N) / 32) * N * 8; }
+constexpr size_t kLsMaxSmem = 200 * 1024;
+
 static int local_search_impl(int step2_mode, const double* bound, int B, int N, int F, int kind, double alpha, int chains, int sweeps,
                                     uint64_t rng_seed, int S, const double* d, const double* w, const double* r,
                                     const double* m, const double* Mj, const double* Kj, const double* maxd,
@@ -770,13 +775,13 @@ static int local_search_impl(int step2_mode, const double* bound, int B, int N, 
   a.chain_ws = p;
   a.chain_stride = chain_bytes_h(N, F);
   if ((p - (char*)workspace) + (int64_t)B * chains * a.chain_stride > workspace_bytes) return NEPTUNE_E_NOMEM;
-  const int threads = N > 128 ? 768 : 256;
-  size_t sm = (size_t)(threads / 32) * N * 8;
+  const int threads = ls_threads(N);
+  size_t sm = ls_row_bytes(N);
   const size_t tables = (size_t)2 * N * N * 8 + (size_t)4 * F * N * 8 + (size_t)3 * F * N * 4 + (size_t)(4 * N + F) * 8 +
                         (size_t)(F + N) * 4 + (size_t)F * N + 64;
   a.use_smem = (threads == 256 && sm + tables <= 72 * 1024) ? 1 : 0;      // 3 blocks per SM must still fit
   if (a.use_smem) sm += tables;
-  if (sm > 200 * 1024) return NEPTUNE_E_SIZE;
+  if (sm > kLsMaxSmem) return NEPTUNE_E_SIZE;
   if (threads == 256)
     NEPTUNE_CUDA_OK(cudaFuncSetAttribute(k_local_search<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
   else
@@ -810,4 +815,10 @@ extern "C" int neptune_disruption_search(int B, int N, int F, int kind, double a
   return local_search_impl(mode, bound, B, N, F, kind, alpha, chains, sweeps, rng_seed, S, d, w, r, m, Mj, Kj, maxd,
                            cost, budget, old, seeds, nullptr, best_c, best_obj, best_flags, workspace,
                            workspace_bytes, stream);
+}
+
+extern "C" int neptune_local_search_fits(int N, int F, int32_t* fits) {
+  if (N <= 0 || F <= 0 || !fits) return NEPTUNE_E_ARG;
+  *fits = ls_row_bytes(N) <= kLsMaxSmem ? 1 : 0;
+  return 0;
 }

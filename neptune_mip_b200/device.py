@@ -360,6 +360,29 @@ def site_greedy(inst: InstanceBatch, max_rounds: int = 0):
     return c, info
 
 
+def site_search(inst: InstanceBatch, c_u8: torch.Tensor, max_rounds: int = 0):
+    """Best-improvement pod-exchange search for the min-delay objective under nearest-pod routing
+    (`neptune_site_search`) from c_u8[B,F,N] (every function with a pod, e.g. `site_greedy`'s placement), at any size.
+    Returns (c uint8[B,F,N], info int32[B,4] = (rounds, adds, exchanges, relocations),
+    obj float64[B,2] = nearest-pod objective at the start and at the end).  max_rounds <= 0: until a round accepts
+    nothing (at most N*F rounds)."""
+    _require_cuda()
+    lib = _lib.load()
+    dev = inst.d.device
+    assert c_u8.shape == (inst.B, inst.F, inst.N) and c_u8.dtype == torch.uint8 and c_u8.is_contiguous()
+    need = C.c_int64()
+    check(lib.neptune_site_search_workspace_bytes(inst.B, inst.N, inst.F, C.byref(need)), "neptune_site_search_workspace_bytes")
+    ws = torch.empty(need.value, dtype=torch.uint8, device=dev)
+    c = torch.empty_like(c_u8)
+    info = torch.empty((inst.B, 4), dtype=torch.int32, device=dev)
+    obj = torch.empty((inst.B, 2), dtype=torch.float64, device=dev)
+    rounds = max_rounds if max_rounds > 0 else inst.N * inst.F
+    check(lib.neptune_site_search(inst.B, inst.N, inst.F, _ptr(inst.d), _ptr(inst.w), _ptr(inst.m), _ptr(inst.Mj),
+                                  _ptr(c_u8), _ptr(c), rounds, _ptr(info), _ptr(obj), _ptr(ws), ws.numel(), _stream()),
+          "neptune_site_search")
+    return c, info, obj
+
+
 def route_two_choice(inst: InstanceBatch, c_u8: torch.Tensor, want_x=True, max_iters=500):
     """Nearest / second-nearest routing with per-node shares lowered until the CPU rows hold (`neptune_route_two_choice`):
     the router for sizes the per-instance ones do not reach.  c_u8[B,F,N] ->
@@ -472,13 +495,26 @@ def route_lp(inst: InstanceBatch, c_u8: torch.Tensor, want_x=False, tableau_doub
     return dict(obj=obj, status=status, c_out=c_out, n=n, info=info, x=x)
 
 
+def one_memory_size(inst: InstanceBatch) -> bool:
+    """Every function of an instance needs the same, positive memory: the memory rows are slot counts."""
+    return bool((inst.m == inst.m[:, :1]).all()) and bool((inst.m > 0).all())
+
+
 def lns_supported(inst: InstanceBatch, kind) -> bool:
     """The slot-count search needs a delay term in the objective, one memory size for all functions of an
     instance, and a chain state that fits shared memory."""
     kind = KINDS.get(kind, kind)
     if kind not in (0, 2) or inst.N > 128 or inst.F * inst.N > 4096:
         return False
-    return bool((inst.m == inst.m[:, :1]).all()) and bool((inst.m > 0).all())
+    return one_memory_size(inst)
+
+
+def local_search_fits(N: int, F: int) -> bool:
+    """Whether the add/drop/swap search (`local_search`, `disruption_search`) takes N x F instances
+    (`neptune_local_search_fits`; host arithmetic, no device needed)."""
+    fits = C.c_int32()
+    check(_lib.load().neptune_local_search_fits(N, F, C.byref(fits)), "neptune_local_search_fits")
+    return bool(fits.value)
 
 
 def lns_block_mode(mode: int) -> None:
