@@ -92,11 +92,12 @@ int neptune_assemble_values(int B, int N, int F, int kind, int flags, double alp
 /* ---- (b) PDHG LP relaxation ----------------------------------------------------------------------
  * Replaces the LP work inside `pywraplp.Solver.Solve()` (`core/solvers/solver.py:37`).
  * Diagonally preconditioned, restarted, averaged PDHG on  min obj.x  s.t. lo <= A x <= hi,
- * lb <= x <= ub, for B same-pattern instances at once. */
+ * lb <= x <= ub, for B same-shaped instances at once.  The entry points below never store A: they
+ * regenerate its coefficients from the instance arrays. */
 typedef struct neptune_pdhg_params {
   int     max_iters;        /* hard cap on PDHG iterations */
   int     check_every;      /* iterations between KKT evaluations / restart decisions */
-  int     ruiz_iters;       /* Ruiz equilibration passes (then one Pock-Chambolle pass) */
+  int     ruiz_iters;       /* unused; pass 0 */
   int     reserved;         /* 0.  neptune_pdhg_mf_solve reads it as switches for measurements and tests:
                              * bit 0 = force the 8-byte iteration pass, bits 4..6 = tool diagnostics,
                              * bits 8..10 = rows of a warp in flight (0 = default), bit 11 = register passes whatever the
@@ -122,34 +123,14 @@ typedef struct neptune_pdhg_result {  /* one per instance, written to device mem
   int32_t pad;
 } neptune_pdhg_result;
 
-/* bytes of device workspace neptune_pdhg_solve needs */
-int neptune_pdhg_workspace_bytes(int B, int64_t rows, int64_t cols, int64_t nnz, int64_t* bytes);
-
-/* x[B][cols], y[B][rows] in/out (warm start; zero them for a cold start). */
-int neptune_pdhg_solve(int B, int64_t rows, int64_t cols, int64_t nnz,
-                       const int64_t* row_ptr, const int32_t* col_idx, const double* val,
-                       const int64_t* rowT_ptr, const int32_t* colT_idx, const double* valT,
-                       const double* obj, const double* lo, const double* hi,
-                       const double* col_lb, const double* col_ub,
-                       const neptune_pdhg_params* params_h,
-                       double* x, double* y, neptune_pdhg_result* result_d,
-                       void* workspace, int64_t workspace_bytes, void* stream);
-
-/* The two SpMV building blocks on their own (tests, roofline measurement):
- * out[B][rows] = A x   and   out[B][cols] = A^T y  for B same-pattern instances. */
-int neptune_spmv(int B, int64_t rows, int64_t cols, const int64_t* row_ptr, const int32_t* col_idx,
-                 const double* val, const double* x, double* out, void* stream);
-int neptune_spmv_t(int B, int64_t rows, int64_t cols, const int64_t* rowT_ptr,
-                   const int32_t* colT_idx, const double* valT, const double* y, double* out,
-                   void* stream);
-
-/* ---- (b, matrix-free) the same PDHG without the matrix ----------------------------------------------
+/* ---- (b, matrix-free) PDHG without the matrix -------------------------------------------------------
  * The LP relaxation of the STRENGTHENED min-delay model (what neptune_assemble_* builds with kind =
  * NEPTUNE_KIND_MIN_DELAY, flags = NEPTUNE_FLAG_STRENGTHEN: rows of `neptune/utils/constraints_step1.py:5-65`
- * with the C1a rows free, plus x[i,f,j] <= c[f,j] and x <= 1; objective `objectives.py:4-11`), solved by the
- * algorithm of neptune_pdhg_solve with ruiz_iters = 0 (Pock-Chambolle step sizes), but every coefficient is
- * regenerated from d, w, r, m instead of being read from CSR arrays: one streaming pass over x / yS and their
- * running sums per iteration.  x[B][cols], y[B][rows] are the canonical vectors of that model (in/out, warm
+ * with the C1a rows free, plus x[i,f,j] <= c[f,j] and x <= 1; objective `objectives.py:4-11`), solved with
+ * Pock-Chambolle diagonal step sizes (1 / sum_i |A_ij| per column times eta / omega, 1 / sum_j |A_ij| per non-free
+ * row times eta * omega; eta = 0.99, omega the primal weight) and PDLP's KKT restart criteria (csrc/pdhg_ctl.cuh).
+ * Every coefficient is regenerated from d, w, r, m instead of being read from CSR arrays: one streaming pass over
+ * x / yS and their running sums per iteration.  x[B][cols], y[B][rows] are the canonical vectors of that model (in/out, warm
  * start; the multipliers of the free C1a rows are returned as 0).  Other kinds return NEPTUNE_E_ARG. */
 int neptune_pdhg_mf_workspace_bytes(int B, int N, int F, int64_t* bytes);
 /* host-only: tile geometry of the passes for (B, N, F); out[16] (see csrc/pdhg_mf.cu) */

@@ -40,8 +40,6 @@ _SIGNATURES = {
     "neptune_model_sizes": [_i, _i, _i, _i, C.POINTER(_i64), C.POINTER(_i64), C.POINTER(_i64)],
     "neptune_assemble_pattern": [_i, _i, _i, _i, _p, _p, _p, _p, _p],
     "neptune_assemble_values": [_i, _i, _i, _i, _i, _d] + _INST + [_p] * 9 + [_p],
-    "neptune_pdhg_workspace_bytes": [_i, _i64, _i64, _i64, C.POINTER(_i64)],
-    "neptune_pdhg_solve": [_i, _i64, _i64, _i64] + [_p] * 11 + [C.POINTER(PdhgParams)] + [_p] * 3 + [_p, _i64, _p],
     "neptune_pdhg_mf_workspace_bytes": [_i, _i, _i, C.POINTER(_i64)],
     "neptune_pdhg_mf_geometry": [_i, _i, _i, C.POINTER(C.c_int32)],
     "neptune_pdhg_mf_solve_util": [_i, _i, _i, _i] + [_p] * 7 + [_d, _d, _p] + [C.POINTER(PdhgParams)] + [_p] * 3 + [_p, _i64, _p],
@@ -50,8 +48,6 @@ _SIGNATURES = {
     "neptune_pdhg_mf_column_sums": [_i, _i, _i] + [_p] * 9 + [_p, _i64, _p],
     "neptune_pdhg_mf_local_step": [_i, _i, _i] + [_p] * 3 + [_d, _d, _i, _i] + [_p] * 6 + [_p, _i64, _p, _p],
     "neptune_pdhg_mf_pass": [_i, _i, _i] + [_p] * 6 + [_d, _d, _d, _i, _i] + [_p] * 6 + [_p, _i64, _p, _p],
-    "neptune_spmv": [_i, _i64, _i64, _p, _p, _p, _p, _p, _p],
-    "neptune_spmv_t": [_i, _i64, _i64, _p, _p, _p, _p, _p, _p],
     "neptune_check_solution": [_i, _i, _i, _d] + _INST + [_p] * 5 + [_p],
     "neptune_route_placements": [_i, _i, _i, _p, _p, _p, _p, _p],
     "neptune_route_capacitated": [_i, _i, _i] + [_p] * 10 + [_p],

@@ -1,6 +1,6 @@
-"""Batched solve path: B same-shaped instances through the LP relaxation (PDHG: matrix-free for the min-delay
-model, assembly + CSR otherwise) -> EFTTC -> local search (or, for the min-delay model at sizes the searches with
-shared-memory chain state do not take, greedy -> pod-exchange search -> two-choice routing) -> exact check in one go (what bench.py times, and what a sweep like BASELINE.json's config 5 calls)."""
+"""Batched solve path: B same-shaped instances through the LP relaxation (matrix-free PDHG, all three objectives)
+-> EFTTC -> local search (or, for the min-delay model at sizes the searches with shared-memory chain state do not take,
+greedy -> pod-exchange search -> two-choice routing) -> exact check in one go (what bench.py times, and what a sweep like BASELINE.json's config 5 calls)."""
 from __future__ import annotations
 
 import os
@@ -25,7 +25,6 @@ class BatchParams:
     alpha: float = 0.5
     lp_iters: int = 2048          # PDHG iterations on the strengthened relaxation (bound + rounding guide)
     lp_check_every: int = 256
-    lp_path: str = "auto"         # "auto": matrix-free PDHG (all three objectives); "csr": the assembled model through the CSR solver
     chains: int = 16              # local-search chains per instance (add/drop/swap search)
     sweeps: int = 200
     rng_seed: int = 1
@@ -63,7 +62,7 @@ class BatchResult:
     pdhg_iters: int = 0
     model_dims: tuple = (0, 0, 0)
     pdhg_bytes_per_iter: int = 0  # algorithmic bytes one PDHG iteration of the whole batch moves (DESIGN.md section 3b)
-    pdhg_path: str = ""           # "matrix-free" | "csr"
+    pdhg_path: str = ""           # "matrix-free" when the LP ran
     search_path: str = ""         # "lns" | "local" | "site"
     lns_round: Optional[torch.Tensor] = None     # [B] round at which the returned placement was recorded by its chain
     lns_ms: float = 0.0
@@ -86,32 +85,21 @@ def solve_batch(inst: device.InstanceBatch, prm: BatchParams, time_pdhg: bool = 
     if prm.lp_iters > 0:
         N, F, B = inst.N, inst.F, inst.B
         X = F * N * N
+        # the relaxation is solved matrix-free (nothing is assembled; every coefficient of the strengthened model is
+        # regenerated from d, w, r, m inside the iteration kernels); the models with node columns n[j] add O(N) rows
+        # and columns that live in the small-vector kernel (neptune_pdhg_mf_solve_util)
+        kk = KINDS.get(kind, kind)
+        rows, cols, nnz = device.model_sizes(N, F, kk, FLAG_STRENGTHEN)
         if time_pdhg:
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        if prm.lp_path != "csr":
-            # the relaxation is solved matrix-free (nothing is assembled; every coefficient of the strengthened model is
-            # regenerated from d, w, r, m inside the iteration kernels); the models with node columns n[j] add O(N) rows
-            # and columns that live in the small-vector kernel (neptune_pdhg_mf_solve_util)
-            kk = KINDS.get(kind, kind)
-            rows, cols, nnz = device.model_sizes(N, F, kk, FLAG_STRENGTHEN)
-            if time_pdhg:
-                e0.record()
-            xs, ys, lp_res = device.pdhg_mf_solve(inst_lp, max_iters=prm.lp_iters, check_every=prm.lp_check_every,
-                                                  eps_rel=1e-6, eps_abs=1e-9, kind=kk, alpha=prm.alpha, node_cut=prm.lp_cut)
-            lam0 = ys[:, 3 * F * N + N:3 * F * N + 2 * N].contiguous()       # duals of the CPU rows C4
-            if kk == 2:      # the combined objective scales the delays: prices back in delay units for the search
-                a_d = objective_weights(inst, kind, prm.alpha)[0]
-                lam0 = lam0 / torch.where(a_d > 0, a_d, torch.ones_like(a_d))[:, None]
-            bytes_iter, path = B * (64 * X + 112 * F * N + 8 * N * N), "matrix-free"
-        else:
-            lp = device.assemble(inst, kind, prm.alpha, flags=FLAG_STRENGTHEN)
-            rows, cols, nnz = lp.rows, lp.cols, lp.nnz
-            if time_pdhg:
-                e0.record()
-            xs, ys, lp_res = device.pdhg_solve(lp, max_iters=prm.lp_iters, check_every=prm.lp_check_every,
-                                               eps_rel=1e-6, eps_abs=1e-9)
-            bytes_iter, path = B * (16 * nnz + 88 * cols + 72 * rows) + 8 * nnz + 8 * (rows + cols + 2), "csr"
-            del lp
+            e0.record()
+        xs, ys, lp_res = device.pdhg_mf_solve(inst_lp, max_iters=prm.lp_iters, check_every=prm.lp_check_every,
+                                              eps_rel=1e-6, eps_abs=1e-9, kind=kk, alpha=prm.alpha, node_cut=prm.lp_cut)
+        lam0 = ys[:, 3 * F * N + N:3 * F * N + 2 * N].contiguous()       # duals of the CPU rows C4
+        if kk == 2:      # the combined objective scales the delays: prices back in delay units for the search
+            a_d = objective_weights(inst, kind, prm.alpha)[0]
+            lam0 = lam0 / torch.where(a_d > 0, a_d, torch.ones_like(a_d))[:, None]
+        bytes_iter, path = B * (64 * X + 112 * F * N + 8 * N * N), "matrix-free"
         if time_pdhg:
             e1.record()
             e1.synchronize()

@@ -1,5 +1,5 @@
-// pdhg_ctl.cuh -- per-instance control block of the restarted PDHG solvers (pdhg.cu: CSR matrix;
-// pdhg_mf.cu: matrix-free) and the one-thread-per-instance kernels that take the restart / termination
+// pdhg_ctl.cuh -- per-instance control block of the restarted matrix-free PDHG (pdhg_mf.cu; its numpy statement
+// is tests/mf_reference.solve_ctl) and the one-thread-per-instance kernels that take the restart / termination
 // decisions on the device (PDLP's KKT-error criteria).  Step sizes, restart flags and convergence live in
 // device memory so that the iteration kernels can be replayed from a CUDA graph.
 #pragma once

@@ -1,6 +1,6 @@
 // pdhg_mf.cu -- (b) MATRIX-FREE restarted, averaged, diagonally preconditioned PDHG for the LP relaxation
 // of the strengthened min-delay placement model (same LP as assemble.cu builds with
-// NEPTUNE_FLAG_STRENGTHEN, same algorithm and control logic as pdhg.cu with ruiz_iters = 0).
+// NEPTUNE_FLAG_STRENGTHEN; Pock-Chambolle step sizes, restart / termination control of pdhg_ctl.cuh).
 //
 // Replaces the LP work inside pywraplp.Solver.Solve() (reference core/solvers/solver.py:37) for the model
 // of neptune/utils/constraints_step1.py:5-65 + objectives.py:4-11.  Every coefficient of that model is a
@@ -21,8 +21,8 @@
 // k_mf_small: the F*N-sized updates -- duals y1/y3/y4 from the partial sums (POST), then the c columns of the
 //   next iteration (PREC) and the C2 dual (Y2).
 // Algorithmic bytes per iteration and instance: X*(8 x + 8 yS + 8 xsum + 8 ysum read, the same written)
-//   = 64*X, + 112*F*N (small vectors) + 8*N*N (d, re-read per function from L1/L2)  [X = F*N*N]; the CSR solver
-//   moves 16*nnz + 88*cols + 72*rows ~ 260*X for the same iteration.
+//   = 64*X, + 112*F*N (small vectors) + 8*N*N (d, re-read per function from L1/L2)  [X = F*N*N]; the same iteration
+//   on the assembled CSR matrix moves 16*nnz + 88*cols + 72*rows ~ 260*X.
 //
 // Three iteration passes, all parity-tested against the numpy statement: tests/test_pdhg_mf_gpu.py up to 70 x 3 and
 // 50 x 10; tests/test_pdhg_mf_wide_gpu.py at the branches only wide shapes take, each case pinned to its branch by
@@ -705,8 +705,8 @@ k_mf_eval_small(MfGeo G, MfIn in, MfSt st, Ctl* __restrict__ ctl, int which) {
 }
 
 // ---------------------------------------------------------------------------------------------------
-// setup: step-size vectors S4, S2, the norms behind omega0 and the tolerances (same definitions as k_norms
-// of pdhg.cu), multipliers of the free C1a rows zeroed.
+// setup: step-size vectors S4, S2, the norms behind omega0 and the tolerances (the definitions mf_reference.Generic
+// states on the assembled matrix), multipliers of the free C1a rows zeroed.
 // ---------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_mf_wsum(int N, int64_t n_rows, const double* __restrict__ w,
                                                  double* __restrict__ wsum) {

@@ -163,50 +163,9 @@ def assemble(inst: InstanceBatch, kind, alpha=0.5, flags=0, with_transpose=True)
                  val, valT, obj, lo, hi, col_lb, col_ub, col_int, wmax)
 
 
-def spmv(mdl: Model, x: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    lib = _lib.load()
-    if out is None:
-        out = torch.empty((mdl.B, mdl.rows), dtype=torch.float64, device=x.device)
-    check(lib.neptune_spmv(mdl.B, mdl.rows, mdl.cols, _ptr(mdl.row_ptr), _ptr(mdl.col_idx), _ptr(mdl.val),
-                           _ptr(x), _ptr(out), _stream()), "neptune_spmv")
-    return out
-
-
-def spmv_t(mdl: Model, y: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    lib = _lib.load()
-    if out is None:
-        out = torch.empty((mdl.B, mdl.cols), dtype=torch.float64, device=y.device)
-    check(lib.neptune_spmv_t(mdl.B, mdl.rows, mdl.cols, _ptr(mdl.rowT_ptr), _ptr(mdl.colT_idx), _ptr(mdl.valT),
-                             _ptr(y), _ptr(out), _stream()), "neptune_spmv_t")
-    return out
-
-
 _PDHG_DTYPE = np.dtype([("primal_obj", "f8"), ("dual_obj", "f8"), ("primal_res", "f8"), ("dual_res", "f8"),
                         ("gap", "f8"), ("step", "f8"), ("primal_weight", "f8"), ("iters", "i4"),
                         ("restarts", "i4"), ("converged", "i4"), ("pad", "i4")])
-
-
-def pdhg_solve(mdl: Model, max_iters=20000, check_every=64, eps_rel=1e-6, eps_abs=1e-8, ruiz_iters=10,
-               x0: Optional[torch.Tensor] = None, y0: Optional[torch.Tensor] = None, workspace=None):
-    """Returns (x[B,cols], y[B,rows], results: numpy structured array of length B)."""
-    lib = _lib.load()
-    dev = mdl.val.device
-    x = torch.zeros((mdl.B, mdl.cols), dtype=torch.float64, device=dev) if x0 is None else x0
-    y = torch.zeros((mdl.B, mdl.rows), dtype=torch.float64, device=dev) if y0 is None else y0
-    need = C.c_int64()
-    check(lib.neptune_pdhg_workspace_bytes(mdl.B, mdl.rows, mdl.cols, mdl.nnz, C.byref(need)),
-          "neptune_pdhg_workspace_bytes")
-    if workspace is None or workspace.numel() < need.value:
-        workspace = torch.empty(need.value, dtype=torch.uint8, device=dev)
-    res = torch.zeros(mdl.B * _PDHG_DTYPE.itemsize, dtype=torch.uint8, device=dev)
-    prm = PdhgParams(max_iters, check_every, ruiz_iters, 0, eps_rel, eps_abs)
-    check(lib.neptune_pdhg_solve(mdl.B, mdl.rows, mdl.cols, mdl.nnz, _ptr(mdl.row_ptr), _ptr(mdl.col_idx),
-                                 _ptr(mdl.val), _ptr(mdl.rowT_ptr), _ptr(mdl.colT_idx), _ptr(mdl.valT),
-                                 _ptr(mdl.obj), _ptr(mdl.lo), _ptr(mdl.hi), _ptr(mdl.col_lb), _ptr(mdl.col_ub),
-                                 C.byref(prm), _ptr(x), _ptr(y), _ptr(res), _ptr(workspace),
-                                 workspace.numel(), _stream()), "neptune_pdhg_solve")
-    out = np.frombuffer(res.cpu().numpy().tobytes(), dtype=_PDHG_DTYPE)
-    return x, y, out
 
 
 def objective_weights(inst: InstanceBatch, kind, alpha=0.5):

@@ -1,4 +1,5 @@
-"""numpy prototype of the PDHG variant implemented in csrc/pdhg.cu (for tuning on CPU)."""
+"""Historical numpy prototype of the round-1 PDHG on the assembled CSR matrix (csrc/pdhg.cu, since retired in favour
+of the matrix-free solver, DESIGN.md section 3(b')); kept as the record of how its Ruiz scaling and restarts were tuned."""
 import sys, time
 sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tests')
 import numpy as np, scipy.sparse as sp

@@ -45,7 +45,8 @@ def strengthened(a, kind="min_delay", alpha=0.5, bigm=None):
 
 
 def pc_diag(m):
-    """T = 1/colsum|A|, S = 1/rowsum|A| over the non-free rows (what pdhg.cu does with ruiz_iters = 0)."""
+    """T = 1/colsum|A|, S = 1/rowsum|A| over the non-free rows: the Pock-Chambolle step sizes csrc/pdhg_mf.cu
+    generates in closed form."""
     A = abs(m["A"]).tocsr()
     free = np.isinf(m["lo"]) & np.isinf(m["hi"])
     A = sp.diags((~free).astype(float)) @ A
@@ -54,7 +55,8 @@ def pc_diag(m):
 
 
 class Generic:
-    """PDHG on the CSR matrix, the control logic of pdhg.cu (k_ctl_decide / k_ctl_after_restart)."""
+    """The PDHG iteration on a CSR matrix with the step sizes of `pc_diag` (step and KKT pieces in the form the
+    control logic of csrc/pdhg_ctl.cuh, k_ctl_decide / k_ctl_after_restart, reads them)."""
 
     def __init__(self, m, T, S):
         self.m, self.A, self.At, self.T, self.S = m, m["A"].tocsr(), m["A"].T.tocsr(), T, S
@@ -313,7 +315,7 @@ class MatrixFreeN(MatrixFree):
 
 
 def solve(mf: MatrixFree, max_iters=20000, check=64, eps=1e-6, verbose=False):
-    """restart logic of pdhg.cu on the matrix-free state"""
+    """restart logic of csrc/pdhg_ctl.cuh (k_ctl_decide / k_ctl_after_restart) on the matrix-free state"""
     sums = [np.zeros_like(t) for t in mf.state()]
     rst = [np.array(t) for t in mf.state()]
     diag = None

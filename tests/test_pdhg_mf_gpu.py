@@ -1,12 +1,13 @@
 """(b) matrix-free PDHG (`neptune_pdhg_mf_solve`): the kernels reproduce the numpy statement of the iteration
-(tests/mf_reference.py, proven equal to the CSR iteration on the oracle's matrix in tests/test_mf_reference.py),
-agree with the CSR solver on the assembled matrix, and reach the HiGHS LP optimum."""
+(tests/mf_reference.py, proven equal to the CSR iteration on the strengthened oracle matrix in
+tests/test_mf_reference.py), that matrix is exactly the one the device assembles in the solver's canonical layout,
+and the solver reaches the HiGHS LP optimum."""
 import ctypes
 
 import numpy as np
 import pytest
 
-from helpers import arrays_of, cuda_batch, float_payload
+from helpers import KIND_NAMES, arrays_of, cuda_batch, float_payload
 from mf_reference import MatrixFree, MatrixFreeN, node_cut_bigm, run_fixed, solve, strengthened
 from neptune_mip_b200 import synth
 from oracle import mip as omip
@@ -137,19 +138,28 @@ def test_bulk_copy_pass_frozen_instances_and_solo_runs(mode, unfused):
         assert np.array_equal(y[b].cpu().numpy(), ys[0].cpu().numpy())
 
 
-def test_agrees_with_the_csr_solver_on_the_assembled_matrix():
-    """same algorithm on the assembled (reference-identical + strengthening rows) CSR matrix with the same step
-    sizes (ruiz_iters = 0).  Bound 5e-5 relative (BASELINE.json's 1e-4 with margin): the CSR kernels square a
-    reciprocal square root where the closed form divides, and sum every row in another order"""
+def test_strengthened_assembly_equals_the_reference_statement():
+    """the strengthened model the device assembles (`assemble(..., flags=FLAG_STRENGTHEN)`: the model whose canonical
+    x / y vectors the matrix-free solver reads and writes) IS the matrix of `mf_reference.strengthened`, on which
+    tests/test_mf_reference.py proves the numpy matrix-free iteration equal to the CSR iteration.  Exact equality of
+    the pattern, the values, the row and column bounds and the objective, for all three objectives at 20x5 and 8x4,
+    three instances in one batch each"""
     from neptune_mip_b200 import device
     from neptune_mip_b200._lib import FLAG_STRENGTHEN
-    inst = cuda_batch([synth.random_payload(20, 5, s, node_cores=100) for s in range(3)])
-    mdl = device.assemble(inst, "min_delay", flags=FLAG_STRENGTHEN)
-    xa, ya, ra = device.pdhg_solve(mdl, max_iters=64, check_every=64, ruiz_iters=0, eps_rel=1e-13, eps_abs=1e-15)
-    xb, yb, rb = device.pdhg_mf_solve(inst, max_iters=64, check_every=64, eps_rel=1e-13, eps_abs=1e-15)
-    assert _close(xb.cpu().numpy(), xa.cpu().numpy(), 5e-5) and _close(yb.cpu().numpy(), ya.cpu().numpy(), 5e-5)
-    assert np.allclose(ra["primal_obj"], rb["primal_obj"], rtol=5e-5)
-    print("csr vs matrix-free after 64 iterations: max |dx| %.2e, max |dy| %.2e" % (float((xa - xb).abs().max()), float((ya - yb).abs().max())))
+    for (N, F), cores in (((20, 5), 100), ((8, 4), 30)):
+        payloads = [synth.random_payload(N, F, s, node_cores=cores) for s in range(3)]
+        inst = cuda_batch(payloads)
+        for kind in KIND_NAMES:
+            mdl = device.assemble(inst, kind, 0.5, flags=FLAG_STRENGTHEN)
+            for b, p in enumerate(payloads):
+                ref = strengthened(arrays_of(p), kind, 0.5)
+                A, case = ref["A"], (N, F, kind, b)
+                assert (mdl.rows, mdl.cols, mdl.nnz) == (A.shape[0], A.shape[1], A.nnz), case
+                assert np.array_equal(mdl.row_ptr.cpu().numpy(), A.indptr), case
+                assert np.array_equal(mdl.col_idx.cpu().numpy(), A.indices), case
+                assert np.array_equal(mdl.val[b].cpu().numpy(), A.data), case
+                for got, key in ((mdl.lo, "lo"), (mdl.hi, "hi"), (mdl.obj, "obj"), (mdl.col_lb, "lb"), (mdl.col_ub, "ub")):
+                    assert np.array_equal(got[b].cpu().numpy(), ref[key]), (key,) + case
 
 
 @pytest.mark.parametrize("shape,cores", [((12, 5), 25), ((8, 4), 12), ((10, 3), 20)])
@@ -214,11 +224,10 @@ def test_node_variable_models_iterates_equal_the_numpy_reference(name, make, ite
 
 
 @pytest.mark.parametrize("kind", ["min_util", "min_delay_util"])
-def test_node_variable_models_reach_the_highs_lp_optimum_and_the_csr_solver(kind):
-    """LP value of the reference's relaxation with node columns: HiGHS on the oracle's matrix, the CSR solver on the
-    assembled matrix, and the matrix-free solver agree to 1e-4 relative."""
+def test_node_variable_models_reach_the_highs_lp_optimum(kind):
+    """LP value of the reference's relaxation with node columns: HiGHS on the oracle's matrix and the matrix-free
+    solver agree to 1e-4 relative."""
     from neptune_mip_b200 import device
-    from neptune_mip_b200._lib import FLAG_STRENGTHEN
     p = synth.random_payload(12, 5, 1, node_cores=25)
     lp = omip.solve_model(strengthened(arrays_of(p), kind, 0.5), relax=True)
     inst = cuda_batch([p])
@@ -226,9 +235,6 @@ def test_node_variable_models_reach_the_highs_lp_optimum_and_the_csr_solver(kind
     assert res[0]["converged"] == 1
     tol = 1e-4 * (1 + abs(lp["objective"]))
     assert abs(res[0]["primal_obj"] - lp["objective"]) <= tol and abs(res[0]["dual_obj"] - lp["objective"]) <= tol
-    mdl = device.assemble(inst, kind, 0.5, flags=FLAG_STRENGTHEN)
-    xa, ya, ra = device.pdhg_solve(mdl, max_iters=60000, check_every=128, eps_rel=1e-6, eps_abs=1e-9)
-    assert abs(ra[0]["primal_obj"] - res[0]["primal_obj"]) <= 2 * tol
     n = x[0, -inst.N:].cpu().numpy()
     assert n.min() >= 0.0 and n.max() <= 1.0
 

@@ -1,7 +1,8 @@
-"""GPU experiment: matrix-free PDHG (neptune_pdhg_mf_solve) against the CSR solver (neptune_pdhg_solve with
-ruiz_iters = 0, i.e. the same Pock-Chambolle step sizes) -- iterate equality after a fixed number of
-iterations, converged objectives, and time per iteration / achieved GB/s at C2 (batch), C3 and the per-GPU
-share of C4.  Writes gpurun_out/mf_check.json.   python tools/mf_check.py [--quick] [--profile]"""
+"""GPU experiment: the passes of the matrix-free PDHG (neptune_pdhg_mf_solve) against each other -- time per
+iteration, achieved GB/s and iterate differences of the register, pair and bulk-copy passes at C2 (batch), C3, the
+per-GPU share of C4 and C5; the small-vector kernel alone; plain copy ceilings; iterations to 1e-6 on C2 (the bulk
+mode also writes its rows to mf_bulk.json).
+    python tools/mf_check.py [--variants] [--small-phases] [--bulk-diag] [--bulk] [--ceiling] [--converge]"""
 import json
 import os
 import sys
