@@ -62,13 +62,13 @@ __device__ __forceinline__ uint64_t lns_next(uint64_t& s) { s ^= s >> 12; s ^= s
 // ---- shared-memory layout -----------------------------------------------------------------------------------
 // block: dT[N][N] (delay, transposed: the hot loops fix a destination j and run the lanes over sources i),
 //        w[F][N], r[F][N], K[N], slots[N]
-// warp : lam[N] | loadfx[N] | bestv[F*N] | scratch (costT | cur | nxt  /  th  /  exception list) | ints | bytes
+// warp : lam[N] | loadfx[N] | bestv[F*N] | scratch (costT | dp  /  th  /  exception list) | ints | bytes
 __host__ __device__ inline size_t lns_block_shared(int N, int F) {
   return ((size_t)N * N + 2 * (size_t)F * N + (size_t)N) * 8 + (size_t)N * 4 + 64;
 }
 __host__ __device__ inline size_t lns_scratch_bytes(int N, int F, int k, int smax, int maxslots) {
   const size_t fn = (size_t)F * N, nT = (size_t)1 << k, tn = (size_t)(maxslots < F ? maxslots : F) * N;
-  size_t dp = (size_t)F * nT * 8 + 2 * (size_t)smax * 8;      // costT, cur, nxt
+  size_t dp = (size_t)F * nT * 8 + (size_t)smax * 8;          // costT, dp (updated in place, one function at a time)
   size_t th = tn * 4 + tn * 2;                                // thresholds (float) + their scan list (u16) of one node's sources
   if (th < fn * 2) th = fn * 2;                               // exception list (u16)
   return ((dp > th ? dp : th) + 15) & ~(size_t)15;
@@ -80,7 +80,7 @@ __host__ __device__ inline size_t lns_warp_shared(int N, int F, int k, int smax,
   b += (size_t)N * 8;               // loadfx
   b += (fn * 4 + 15) & ~(size_t)15; // bestv (float: it ranks candidates, the records are priced exactly afterwards)
   b += lns_scratch_bytes(N, F, k, smax, maxslots);
-  b += ((size_t)F + 64 + (size_t)F) * 4;   // npods, misc (J, rad, mul, incT), fl
+  b += ((size_t)F + 33 + (size_t)F) * 4;   // npods, misc (J, rad, mul, incT, number of states), fl
   b += 3 * fn;                      // asg, c, podlist
   b += (size_t)F * smax;            // choice
   b += (size_t)smax + 2 * (size_t)F + 16;  // supp table, oldT, newT
@@ -169,13 +169,12 @@ __global__ void __launch_bounds__(WPB * 32, 2) k_lns(LnsArgs a) {
   float* bestv = (float*)wp; wp += ((size_t)fn * 4 + 15) & ~(size_t)15;
   unsigned char* scratch = wp; wp += lns_scratch_bytes(N, F, KK, smax, a.maxslots);
   double* costT = (double*)scratch;                       // [F][NT]
-  double* cur = costT + (size_t)F * NT;
-  double* nxt = cur + smax;
+  double* dp = costT + (size_t)F * NT;                    // [smax]
   float* th = (float*)scratch;                            // aliases the DP arrays (never live together)
   unsigned short* thl = (unsigned short*)(scratch + (size_t)(a.maxslots < F ? a.maxslots : F) * N * 4);   // sources whose threshold needs a pod scan
   unsigned short* exl = (unsigned short*)scratch;         // exception list, ditto
   int* npods = (int*)wp; wp += (size_t)F * 4;
-  int* misc = (int*)wp; wp += 64 * 4;
+  int* misc = (int*)wp; wp += 33 * 4;
   int* fl = (int*)wp; wp += (size_t)F * 4;
   uint8_t* asg = wp; wp += fn;
   uint8_t* c = wp; wp += fn;
@@ -597,35 +596,58 @@ __global__ void __launch_bounds__(WPB * 32, 2) k_lns(LnsArgs a) {
       #pragma unroll 1
       for (int q = 0; q < kk; ++q) if ((s / mul[q]) % rad[q] > 0) supp |= 1 << q;
       suppT[s] = (uint8_t)supp;
-      cur[s] = s == 0 ? 0.0 : INFINITY;
+      dp[s] = s == 0 ? 0.0 : INFINITY;
     }
     __syncwarp();
-    double* pc = cur; double* pn = nxt;
+    // one array, updated in place: state s2 reads only states s2 - inc(T) <= s2, so the states are processed in
+    // descending blocks of 32 and every lane has read before any lane stores its block -- the reads see the values
+    // of the previous function exactly as with two arrays
+    int mulr[KK];                                       // slot increment of each node (k = 4 candidate loop)
+#pragma unroll
+    for (int q = 0; q < KK; ++q) mulr[q] = q < kk ? mul[q] : 0;
     #pragma unroll 1
     for (int f = 0; f < F; ++f) {
       const double* ct = costT + f * NT;
       #pragma unroll 1
-      for (int s2 = lane; s2 < S_; s2 += 32) {
-        const int supp = suppT[s2];
+      for (int sb = (S_ - 1) & ~31; sb >= 0; sb -= 32) {
+        const int s2 = sb + lane;
         double best = INFINITY; int bt = 0;
-        int Ts = supp;
-        #pragma unroll 1
-        while (true) {
-          const double v = pc[s2 - incT[Ts]] + ct[Ts];
-          if (v < best) { best = v; bt = Ts; }
-          if (Ts == 0) break;
-          Ts = (Ts - 1) & supp;
+        if (s2 < S_) {
+          // the subsets of the used nodes in descending order (ties keep the largest T)
+          const int supp = suppT[s2];
+          if constexpr (KK == 4) {
+            // all 16 subsets unrolled, increments in registers: the loads of one state do not depend on each other
+            // (measured faster at k = 4; slower at k = 3, where a state has ~5 subsets and the build has 80 registers)
+#pragma unroll
+            for (int T = NT - 1; T >= 0; --T) {
+              if ((T & ~supp) != 0) continue;
+              int inc = 0;
+#pragma unroll
+              for (int q = 0; q < KK; ++q) if ((T >> q) & 1) inc += mulr[q];
+              const double v = dp[s2 - inc] + ct[T];
+              if (v < best) { best = v; bt = T; }
+            }
+          } else {
+            int Ts = supp;
+            #pragma unroll 1
+            while (true) {
+              const double v = dp[s2 - incT[Ts]] + ct[Ts];
+              if (v < best) { best = v; bt = Ts; }
+              if (Ts == 0) break;
+              Ts = (Ts - 1) & supp;
+            }
+          }
         }
-        pn[s2] = best; choice[f * smax + s2] = (uint8_t)bt;
+        __syncwarp();
+        if (s2 < S_) { dp[s2] = best; choice[f * smax + s2] = (uint8_t)bt; }
       }
       __syncwarp();
-      double* t_ = pc; pc = pn; pn = t_;
     }
     // best final state (utilisation: an empty node costs nothing, a used one u)
     double bv = INFINITY; int bs = 0x7fffffff;
     #pragma unroll 1
     for (int s = lane; s < S_; s += 32) {
-      double v = pc[s];
+      double v = dp[s];
       if (u != 0.0) v += u * (double)__popc((unsigned)suppT[s]);
       if (v < bv) { bv = v; bs = s; }
     }
