@@ -288,6 +288,24 @@ int neptune_lns_search(int B, int N, int F, int kind, double alpha, int chains, 
                        const double* guide, const double* lam0, int S, const uint8_t* seeds,
                        int max_slots /* >= max_j floor(Mj / m), or 0 for F: sizes the shared-memory scratch */,
                        uint8_t* out_c, double* out_g, double* out_lb, int32_t* out_round, void* stream);
+/* neptune_lns_search_global: neptune_lns_search with every chain's state in a workspace slab instead of shared memory,
+ * for instances the shared-memory kernel refuses (N > 128 or F*N > 4096; BASELINE configs 3 and 4).  Same arguments and
+ * the same records bit for bit wherever both run (same random streams, evaluation and summation orders, decisions), at
+ * any N <= 65534 with F*N < 2^31; kind 1 is refused (NEPTUNE_E_ARG), larger sizes NEPTUNE_E_SIZE, a workspace smaller
+ * than neptune_lns_search_global_workspace_bytes NEPTUNE_E_NOMEM.  It also returns out_asg[B][2*chains][F][N] (uint16):
+ * the node of each source's nearest priced pod when the record was taken.  A record is taken only with no node
+ * overloaded, so routing every source whole to that pod is a feasible point of the MIP whose delay is the record's
+ * upper bound -- a routing for records too large for neptune_route_lp.  The workspace holds each instance's
+ * transposed delay matrix (8 N^2 bytes) and about 13 F*N bytes per chain. */
+int neptune_lns_search_global(int B, int N, int F, int kind, double alpha, int chains, int rounds, int k,
+                              double noise_coef, uint64_t rng_seed,
+                              const double* d, const double* w, const double* r, const double* m,
+                              const double* Mj, const double* Kj, const double* maxd,
+                              const double* guide, const double* lam0, int S, const uint8_t* seeds, int max_slots,
+                              uint8_t* out_c, double* out_g, double* out_lb, int32_t* out_round, uint16_t* out_asg,
+                              void* workspace, int64_t workspace_bytes, void* stream);
+/* workspace of neptune_lns_search_global (host arithmetic, no device needed) */
+int neptune_lns_search_global_workspace_bytes(int B, int N, int F, int chains, int k, int max_slots, int64_t* bytes);
 /* chains per thread block of neptune_lns_search: 0 (default) = 8 while all blocks are resident at once, 12 (at 80
  * registers) beyond; 1 = always 8; 2 = always 12.  The results do not depend on it (a chain's random stream is a
  * function of its index only); it is a tuning and measurement switch. */

@@ -61,6 +61,8 @@ _SIGNATURES = {
     "neptune_route_two_choice": [_i, _i, _i] + [_p] * 4 + [_p] * 6 + [C.POINTER(C.c_int32), _i, _p, _i64, _p],
     "neptune_lns_block_mode": [_i],
     "neptune_lns_search": [_i, _i, _i, _i, _d, _i, _i, _i, _d, C.c_uint64] + [_p] * 9 + [_i, _p, _i, _p, _p, _p, _p, _p],
+    "neptune_lns_search_global": [_i, _i, _i, _i, _d, _i, _i, _i, _d, C.c_uint64] + [_p] * 9 + [_i, _p, _i] + [_p] * 6 + [_i64, _p],
+    "neptune_lns_search_global_workspace_bytes": [_i, _i, _i, _i, _i, _i, C.POINTER(_i64)],
     "neptune_eval_placements": [_i, _i, _i, _i, _d] + _INST + [_p] * 4 + [_p],
     "neptune_local_search": [_i, _i, _i, _i, _d, _i, _i, C.c_uint64, _i] + _INST + [_p] * 6 + [_p, _i64, _p],
     "neptune_disruption_search": [_i, _i, _i, _i, _d, _i, _p, _i, _i, C.c_uint64, _i] + _INST + [_p] * 5 + [_p, _i64, _p],

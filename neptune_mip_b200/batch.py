@@ -13,7 +13,7 @@ import numpy as np
 import torch
 
 from . import device
-from ._lib import FLAG_STRENGTHEN, KINDS, OK_ALL, OK_C_X, OK_CPU, OK_HANDLE, OK_MEMORY, OK_N_C
+from ._lib import FLAG_STRENGTHEN, KINDS, OK_ALL, OK_C_X, OK_CPU, OK_HANDLE, OK_MEMORY, OK_N_C, NeptuneError
 
 # the checks of the min-delay model: it has no budget row (C6), so the budget flag does not make its answer infeasible
 MIN_DELAY_FLAGS = OK_HANDLE | OK_MEMORY | OK_CPU | OK_C_X | OK_N_C
@@ -30,7 +30,9 @@ class BatchParams:
     rng_seed: int = 1
     search: str = "auto"          # "auto": slot-count LNS (csrc/lns.cu) where it applies, else the add/drop/swap search, and for the
                                   # min-delay model at sizes neither takes (N > 1066) the pod-exchange search; "local": always the
-                                  # add/drop/swap search; "site": always the pod-exchange search (min-delay only)
+                                  # add/drop/swap search; "site": always the pod-exchange search (min-delay only); "lns": the
+                                  # slot-count LNS at every size (kinds 0 and 2, one memory size): beyond shared memory (N > 128 or
+                                  # F*N > 4096) with the chain state in global memory, started from the pod-exchange search's placement
     lp_cut: bool = True           # relax with the Chvatal-Gomory rounding of the memory rows (one memory size per instance)
     lns_chains: int = 96          # warp-sized chains per instance
     lns_fill_waves: bool = False  # raise the chain count (at most 1.5x) until the blocks of the search fill whole waves of the GPU
@@ -73,14 +75,18 @@ def solve_batch(inst: device.InstanceBatch, prm: BatchParams, time_pdhg: bool = 
     kind = prm.kind
     lp_res, guide, lam0, pdhg_ms, iters, dims = None, None, None, 0.0, 0, (0, 0, 0)
     bytes_iter, path = 0, ""
-    use_lns = prm.search == "auto" and device.lns_supported(inst, kind)
-    if use_lns and KINDS.get(kind, kind) == 2 and not bool((objective_weights(inst, kind, prm.alpha)[0] > 0).all()):
+    use_lns = prm.search in ("auto", "lns") and device.lns_supported(inst, kind)
+    delay_term = KINDS.get(kind, kind) != 2 or bool((objective_weights(inst, kind, prm.alpha)[0] > 0).all())
+    if use_lns and not delay_term:
         use_lns = False         # no workload: the combined objective has no delay term (objectives.py:34-35), nothing to price
+    lns_global = prm.search == "lns" and not device.lns_supported(inst, kind)
+    if lns_global and not (delay_term and device.lns_global_supported(inst, kind)):
+        raise ValueError("search='lns' needs a delay term in the objective and one memory size per instance")
     use_site = prm.search == "site" or (prm.search == "auto" and KINDS.get(kind, kind) == 0 and not use_lns
                                         and not device.local_search_fits(inst.N, inst.F))
     if use_site and KINDS.get(kind, kind) != 0:
         raise ValueError("search='site' solves the min-delay model only")
-    cut = prm.lp_cut and (use_lns or (use_site and device.one_memory_size(inst)))
+    cut = prm.lp_cut and (use_lns or lns_global or (use_site and device.one_memory_size(inst)))
     inst_lp = device.slot_relaxation(inst) if cut else inst
     if prm.lp_iters > 0:
         N, F, B = inst.N, inst.F, inst.B
@@ -111,6 +117,13 @@ def solve_batch(inst: device.InstanceBatch, prm: BatchParams, time_pdhg: bool = 
     if use_site:
         best_c, x, n, flags, scores = site_step1(inst, prm.alpha)
         return BatchResult(best_c, x, n, flags, scores, lp_res, pdhg_ms, iters, dims, bytes_iter, path, "site")
+    if lns_global:
+        # the relaxation guides the chains (roundings of c-bar, CPU-row prices) only where it converged everywhere
+        conv = lp_res is not None and bool((lp_res["converged"] != 0).all())
+        best_c, x, n, flags, scores, lns_round, lns_ms, lns_diag = lns_global_step1(
+            inst, kind, prm, guide if conv else None, lam0 if conv else None, time_it=time_pdhg)
+        return BatchResult(best_c, x, n, flags, scores, lp_res, pdhg_ms, iters, dims, bytes_iter, path, "lns",
+                           lns_round, lns_ms, lns_diag)
     cache = {}
 
     def get_seeds():
@@ -177,6 +190,32 @@ def site_step1(inst: device.InstanceBatch, alpha=0.5):
             c[take], x[take], n[take], flags[take], scores[take] = cf[take], xf[take], nf[take], ff[take], sf[take]
         del xf
     return c, x, n, flags, scores
+
+
+def lns_global_step1(inst: device.InstanceBatch, kind, prm: "BatchParams", guide, lam0, time_it=False):
+    """The slot-count search at sizes beyond shared memory (`lns_search_global`).  EFTTC (one block per instance) and the
+    capacity-aware router do not finish at BASELINE config 4, so neither runs: chain 0 starts from the pod-exchange
+    search's placement (`site_greedy` -> `site_search`), the other chains from it too or, with a guide, from roundings
+    of c-bar; records the routing LP cannot price keep the whole-flow routing they were certified with.  The start
+    placement routed by `route_two_choice` is one more candidate: the answer is never worse than it.
+    Returns what `lns_step1` returns."""
+    kk = KINDS.get(kind, kind)
+    M, col = (MIN_DELAY_FLAGS, 0) if kk == 0 else (OK_ALL, 2)
+    cg, _ = device.site_greedy(inst)
+    cs, _, _ = device.site_search(inst, cg)
+    del cg
+    prm = dataclasses.replace(prm, lns_local_chains=0, lns_polish=0)
+    c, x, n, flags, scores, rnd, ms, diag = lns_step1(inst, kind, prm, guide, lam0, cs[:, None].contiguous(), time_it,
+                                                      global_state=True)
+    c2, x2, n2, _, _, _ = device.route_two_choice(inst, cs)
+    f2, s2 = device.check_solution(inst, x2, device.u8_to_f64(c2), n2, prm.alpha)
+    ok, ok2 = (flags & M) == M, (f2 & M) == M
+    take = ok2 & (~ok | (s2[:, col] < scores[:, col]))
+    if bool(take.any()):
+        c[take], x[take], n[take], flags[take], scores[take] = c2[take], x2[take], n2[take], f2[take], s2[take]
+        rnd[take] = -1
+    diag["start_won"] = take
+    return c, x, n, flags, scores, rnd, ms, diag
 
 
 _DEBUG_SYNC = int(os.environ.get("NEPTUNE_DEBUG_SYNC", "0"))
@@ -261,6 +300,16 @@ def polish_exact(inst: device.InstanceBatch, kind, alpha, c: torch.Tensor, max_i
 objective_weights = device.objective_weights      # (a_d[B], a_u[B]) of the three objectives
 
 
+def _route_lp_or_none(inst: device.InstanceBatch, c_u8: torch.Tensor, want_x=False):
+    """`route_lp`, or None where the library refuses the size (F*N > 2^24)"""
+    try:
+        return device.route_lp(inst, c_u8, want_x=want_x)
+    except NeptuneError as e:
+        if "size does not fit" not in str(e):
+            raise
+        return None
+
+
 def fill_waves(B: int, chains: int, chains_per_block: int = 8, resident_blocks: int = 2 * 148, cap: float = 1.5) -> int:
     """Largest chain count with the same number of waves of search blocks (`chains_per_block` chains per block, two
     blocks per SM), at most `cap` times what was asked.  32 instances x 96 chains (384 blocks = 1.3 waves) take as long
@@ -273,9 +322,11 @@ def fill_waves(B: int, chains: int, chains_per_block: int = 8, resident_blocks: 
     return max(chains, min(fit * chains_per_block, int(cap * chains) // chains_per_block * chains_per_block))
 
 
-def lns_step1(inst: device.InstanceBatch, kind, prm: "BatchParams", guide, lam0, seeds, time_it=False):
+def lns_step1(inst: device.InstanceBatch, kind, prm: "BatchParams", guide, lam0, seeds, time_it=False, global_state=False):
     """Slot-count LNS -> exact pricing of the best chain records (routing LP) -> exact routing + checkers of the
-    winner.  Returns (c uint8[B,F,N], x, n, flags, scores, round[B], search ms, diagnostics)."""
+    winner.  Returns (c uint8[B,F,N], x, n, flags, scores, round[B], search ms, diagnostics).  `global_state`: the
+    chains run in `lns_search_global`, and a record the routing LP does not price (tableau too large, or the size
+    refused) is valued and routed by the whole-flow routing its chain certified it with."""
     B, N, F = inst.B, inst.N, inst.F
     if time_it:
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -285,13 +336,16 @@ def lns_step1(inst: device.InstanceBatch, kind, prm: "BatchParams", guide, lam0,
     main_chains = fill_waves(B, prm.lns_chains) if prm.lns_fill_waves else prm.lns_chains
     pops = []                 # populations: dict(c, g, r, other, chains), records [0, chains) by upper bound, [chains, 2 chains) by lower
 
-    def population(chains, n_rounds, k, noise, rng, guide_, seeds_, round_scale=1, round_offset=0):
-        c_, g_, r_ = device.lns_search(inst, kind, prm.alpha, chains, n_rounds, k, noise, rng, guide_, lam0, seeds_)
-        pops.append(dict(c=c_, g=g_, r=r_ * round_scale + round_offset, other=device.lns_search.last_other_bound, chains=chains))
+    search = device.lns_search_global if global_state else device.lns_search
 
-    def records(upper):
+    def population(chains, n_rounds, k, noise, rng, guide_, seeds_, round_scale=1, round_offset=0):
+        out = search(inst, kind, prm.alpha, chains, n_rounds, k, noise, rng, guide_, lam0, seeds_)
+        pops.append(dict(c=out[0], g=out[1], r=out[2] * round_scale + round_offset, other=search.last_other_bound,
+                         chains=chains, asg=out[3] if global_state else None))
+
+    def records(upper, keys=("c", "g", "r", "other")):
         part = lambda t, p: t[:, :p["chains"]] if upper else t[:, p["chains"]:]          # noqa: E731
-        return tuple(torch.cat([part(p[key], p) for p in pops], dim=1) for key in ("c", "g", "r", "other"))
+        return tuple(torch.cat([part(p[key], p) for p in pops], dim=1) for key in keys)
 
     for ph in range(phases):
         noise = prm.lns_noise * (prm.lns_cooling ** ph)
@@ -330,6 +384,12 @@ def lns_step1(inst: device.InstanceBatch, kind, prm: "BatchParams", guide, lam0,
     idx = torch.cat([iu, il + ub_g.shape[1]], dim=1)
     E = idx.shape[1]
     elite = torch.gather(out_c, 1, idx[:, :, None, None].expand(B, E, F, N)).contiguous()
+    if global_state:
+        out_a = torch.cat([records(True, ("asg",))[0], records(False, ("asg",))[0]], dim=1)
+        elite_asg = torch.gather(out_a, 1, idx[:, :, None, None].expand(B, E, F, N))
+        del out_a
+        # the whole-flow value of each elite: the bound of the records by upper bound, the other bound of the others
+        elite_wf = torch.gather(torch.cat([ub_g, lb_u], dim=1), 1, idx)
     if prm.lns_local_chains > 0:
         # one more candidate from the add/drop/swap search (it prices overload by a penalty instead of node prices and
         # does better where most CPU rows bind); restarted from the best records
@@ -339,10 +399,16 @@ def lns_step1(inst: device.InstanceBatch, kind, prm: "BatchParams", guide, lam0,
         elite = torch.cat([elite, lc[:, None]], dim=1).contiguous()
         idx = torch.cat([idx, idx[:, :1]], dim=1)
         E += 1
-    pr = device.route_lp(inst, elite)
+    pr = _route_lp_or_none(inst, elite) if global_state else device.route_lp(inst, elite)
     a_d, a_u = objective_weights(inst, kind, prm.alpha)
+    if pr is None:        # the size is refused: every record keeps its certified whole-flow routing
+        st0 = torch.full((B, E), 2, dtype=torch.int32, device=elite.device)
+        pr = dict(obj=torch.full((B, E), float("inf"), dtype=torch.float64, device=elite.device), status=st0,
+                  n=torch.zeros((B, E, N), dtype=torch.float64, device=elite.device), info=torch.zeros((B, E, 2), dtype=torch.int32, device=elite.device))
     val = a_d[:, None] * pr["obj"] + a_u[:, None] * pr["n"].sum(dim=-1)
     val = torch.where(pr["status"] == 1, val, torch.full_like(val, float("inf")))
+    if global_state:
+        val = torch.where(pr["status"] == 2, elite_wf, val)
     order = torch.argsort(val, dim=1, stable=True)
     ar = torch.arange(B, device=val.device)
     best_c = x = n = flags = scores = rnd = None
@@ -355,25 +421,49 @@ def lns_step1(inst: device.InstanceBatch, kind, prm: "BatchParams", guide, lam0,
         polished, pval = polish_exact(inst, kind, prm.alpha, start, max_iters=abs(prm.lns_polish) if prm.lns_polish else 12)
         if _DEBUG_SYNC:
             torch.cuda.synchronize(); print('polish done', flush=True)
+    # the checks an answer must pass: the min-delay model has no budget row, so at sizes where only the global-state
+    # search runs its answers need not pass the budget check (the shared-memory path keeps asking for all six)
+    M = MIN_DELAY_FLAGS if global_state and KINDS.get(kind, kind) == 0 else OK_ALL
+
+    def certified_routing(pick):
+        """(c, x, n, unrouted[B]) of the picked records' whole-flow routings; a chain that never took a record returns its
+        current routing, where a source may have no pod (node id >= N): such an instance is marked, not routed"""
+        a_ = elite_asg[ar, pick]
+        bad = (a_ >= N).flatten(1).any(dim=1)
+        return (*device.routing_of_assignment(inst, torch.where(bad[:, None, None], torch.zeros_like(a_), a_)), bad)
     for rank in range(E):
         pick = order[:, rank]
         cand = elite[ar, pick].contiguous() if not (rank == 0 and polished is not None) else polished
-        fin = device.route_lp(inst, cand[:, None].contiguous(), want_x=True)
-        cx, cc, cn = fin["x"][:, 0].contiguous(), fin["c_out"][:, 0].contiguous(), fin["n"][:, 0].contiguous()
-        st = fin["status"][:, 0]
-        big = st == 2
-        if bool(big.any()):       # tableau larger than the slab: the heuristic capacity-aware routing stands in
-            hc, hx, hn, _, _ = device.route_capacitated(inst, cand)
-            cc[big], cx[big], cn[big] = hc[big], hx[big], hn[big]
+        if global_state and bool((pr["status"][ar, pick] == 2).all()):
+            fin = None            # no instance would use the exact routing: skip the LP
+        else:
+            fin = _route_lp_or_none(inst, cand[:, None].contiguous(), want_x=True) if global_state else \
+                device.route_lp(inst, cand[:, None].contiguous(), want_x=True)
+        unrouted = None           # instances whose certified routing leaves a source without a pod (no record)
+        if fin is None:
+            cc, cx, cn, unrouted = certified_routing(pick)
+        else:
+            cx, cc, cn = fin["x"][:, 0].contiguous(), fin["c_out"][:, 0].contiguous(), fin["n"][:, 0].contiguous()
+            st = fin["status"][:, 0]
+            big = st == 2
+            if bool(big.any()) and global_state:      # the routing the record was certified with
+                hc, hx, hn, unrouted = certified_routing(pick)
+                cc[big], cx[big], cn[big] = hc[big], hx[big], hn[big]
+                unrouted = unrouted & big
+            elif bool(big.any()):       # tableau larger than the slab: the heuristic capacity-aware routing stands in
+                hc, hx, hn, _, _ = device.route_capacitated(inst, cand)
+                cc[big], cx[big], cn[big] = hc[big], hx[big], hn[big]
         fl, sc = device.check_solution(inst, cx, device.u8_to_f64(cc), cn, prm.alpha)
+        if unrouted is not None:
+            fl = torch.where(unrouted, torch.zeros_like(fl), fl)
         if best_c is None:
             best_c, x, n, flags, scores = cc, cx, cn, fl, sc
             rnd = torch.gather(out_round, 1, torch.gather(idx, 1, pick[:, None]))[:, 0]
         else:
-            take = (flags != OK_ALL) & (fl == OK_ALL)
+            take = ((flags & M) != M) & ((fl & M) == M)
             if bool(take.any()):
                 best_c[take], x[take], n[take], flags[take], scores[take] = cc[take], cx[take], cn[take], fl[take], sc[take]
-        if bool((flags == OK_ALL).all()):
+        if bool(((flags & M) == M).all()):
             break
     ms = 0.0
     if time_it:

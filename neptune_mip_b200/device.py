@@ -468,6 +468,13 @@ def lns_supported(inst: InstanceBatch, kind) -> bool:
     return one_memory_size(inst)
 
 
+def lns_global_supported(inst: InstanceBatch, kind) -> bool:
+    """The slot-count search with its chain state in global memory (`lns_search_global`): a delay term, one memory
+    size per instance, N <= 65534."""
+    kind = KINDS.get(kind, kind)
+    return kind in (0, 2) and inst.N <= 65534 and inst.F * inst.N < 2 ** 31 and one_memory_size(inst)
+
+
 def local_search_fits(N: int, F: int) -> bool:
     """Whether the add/drop/swap search (`local_search`, `disruption_search`) takes N x F instances
     (`neptune_local_search_fits`; host arithmetic, no device needed)."""
@@ -505,6 +512,58 @@ def lns_search(inst: InstanceBatch, kind, alpha=0.5, chains=32, rounds=4000, k=3
           "neptune_lns_search")
     lns_search.last_other_bound = out_lb          # the other end of each record's bracket (diagnostics)
     return out_c, out_g, out_round
+
+
+def lns_search_global_workspace_bytes(B: int, N: int, F: int, chains: int, k: int, max_slots: int) -> int:
+    """Workspace of `lns_search_global` (`neptune_lns_search_global_workspace_bytes`; host arithmetic, no device needed)."""
+    need = C.c_int64()
+    check(_lib.load().neptune_lns_search_global_workspace_bytes(B, N, F, chains, k, max_slots, C.byref(need)),
+          "neptune_lns_search_global_workspace_bytes")
+    return need.value
+
+
+def lns_search_global(inst: InstanceBatch, kind, alpha=0.5, chains=32, rounds=4000, k=3, noise_coef=0.06, rng_seed=1,
+                      guide: Optional[torch.Tensor] = None, lam0: Optional[torch.Tensor] = None,
+                      seeds_u8: Optional[torch.Tensor] = None):
+    """`lns_search` with every chain's state in global memory (`neptune_lns_search_global`): any N <= 65534, and where
+    both run the same records bit for bit.  Returns (c, g, round) as `lns_search` does, plus asg int32[B,2*chains,F,N]:
+    the node each source was routed to, whole, when its chain took the record (no node overloaded: a feasible routing
+    whose delay is the upper bound of entries [:chains])."""
+    lib = _lib.load()
+    kind = KINDS.get(kind, kind)
+    dev = inst.d.device
+    B, N, F = inst.B, inst.N, inst.F
+    S = 0 if seeds_u8 is None else seeds_u8.shape[1]
+    out_c = torch.empty((B, 2 * chains, F, N), dtype=torch.uint8, device=dev)
+    out_g = torch.empty((B, 2 * chains), dtype=torch.float64, device=dev)
+    out_round = torch.empty((B, 2 * chains), dtype=torch.int32, device=dev)
+    out_lb = torch.empty((B, 2 * chains), dtype=torch.float64, device=dev)
+    out_asg = torch.empty((B, 2 * chains, F, N), dtype=torch.int16, device=dev)       # uint16 node ids
+    max_slots = int(torch.floor(inst.Mj / inst.m[:, :1] + 1e-9).max().clamp(min=0, max=F).item())
+    ws = torch.empty(lns_search_global_workspace_bytes(B, N, F, chains, k, max_slots), dtype=torch.uint8, device=dev)
+    check(lib.neptune_lns_search_global(B, N, F, kind, C.c_double(alpha), chains, rounds, k, C.c_double(noise_coef),
+                                        C.c_uint64(rng_seed), _ptr(inst.d), _ptr(inst.w), _ptr(inst.r), _ptr(inst.m),
+                                        _ptr(inst.Mj), _ptr(inst.Kj), _ptr(inst.maxd), _ptr(guide), _ptr(lam0), S,
+                                        _ptr(seeds_u8), max_slots, _ptr(out_c), _ptr(out_g), _ptr(out_lb), _ptr(out_round),
+                                        _ptr(out_asg), _ptr(ws), ws.numel(), _stream()), "neptune_lns_search_global")
+    del ws
+    lns_search_global.last_other_bound = out_lb
+    return out_c, out_g, out_round, out_asg.to(torch.int32) & 0xFFFF
+
+
+def routing_of_assignment(inst: InstanceBatch, asg: torch.Tensor):
+    """asg int[B,F,N] (node of every source) -> (c uint8[B,F,N], x[B,N,F,N], n[B,N]): every source routed whole to its
+    node, only the pods some source uses open."""
+    B, N, F = inst.B, inst.N, inst.F
+    if bool((asg >= N).any()) or bool((asg < 0).any()):
+        raise ValueError("routing_of_assignment: a source without a node (a chain that took no record)")
+    idx = asg.to(torch.int64)
+    c = torch.zeros((B, F, N), dtype=torch.uint8, device=asg.device)
+    c.scatter_(2, idx, 1)
+    x = torch.zeros((B, N, F, N), dtype=torch.float64, device=asg.device)
+    x.scatter_(3, idx.permute(0, 2, 1)[..., None], 1.0)
+    n = (c.amax(dim=1) > 0).to(torch.float64)
+    return c, x, n
 
 
 def slot_relaxation(inst: InstanceBatch) -> InstanceBatch:
